@@ -15,7 +15,11 @@ the canonical figure can exceed the HBM peak; `hbm_gbs_actual_traffic` / `passes
 kernels really move and `roofline` times the dominant kernel against its own bytes.  N > 1: the feature axis is sharded (strong scaling), one NCCL
 all-reduce of the (n x B + B) partial block scores per trip.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
+
+--dump-outputs DIR writes the fitted attributes of the last timed fit as DIR/<name>.npy (see dump_outputs), so that two
+builds can be compared output for output on the same seeded inputs.  With N > 1 GPUs rank 0 writes them, and the
+per-feature attributes (W_, P_, R_, beta_, the scalers) are its shard of the features.
 """
 from __future__ import annotations
 
@@ -60,7 +64,13 @@ def parse():
     ap.add_argument("--parity-features", type=int, default=1024, help="features per block of the dense parity slice (NaN slice: a quarter)")
     ap.add_argument("--seed", type=int, default=20261017)
     ap.add_argument("--verbose", action="store_true")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the fitted attributes of the last timed fit as DIR/<name>.npy "
+                         "(N > 1 GPUs: rank 0 writes, per-feature attributes are its feature shard)")
+    args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    return args
 
 
 VERBOSE = False
@@ -75,6 +85,43 @@ def log(*a):
 def fit_bytes(n, p, K, trips):
     """Canonical algorithmic traffic of one NIPALS fit (SURVEY.md 8d / BASELINE.md section 4)."""
     return 16.0 * n * p * (1 + K + sum(trips))
+
+
+DUMP_BYTES = 64 << 20   # --dump-outputs: at most this much in all
+DUMP_ROWS = 16384       # ... and at first this many rows of an array; halved until the budget holds
+
+
+def dump_outputs(model, out_dir, write=True):
+    """Fitted attributes of `model` -- every array the golden fixtures record (oracle.make_golden.snapshot) and the NIPALS
+    trip counts -- as out_dir/<name>.npy in float64 ("T_/0" -> "T_.0.npy"; integer arrays widened, scalars stored as one
+    element; empty arrays such as the W_concat_ of a fit that never builds it hold nothing to compare and are left out).
+    An array with more rows than the row budget (the per-feature results of the full-size workload) keeps a sorted sample of rows drawn from a
+    generator seeded with its row count, so two builds keep the same rows.  Every rank must call this (materialising the
+    attributes may communicate); only `write` ranks write."""
+    import numpy as np
+    from oracle.make_golden import snapshot
+    with warnings.catch_warnings():
+        warnings.simplefilter("ignore")
+        arrays = snapshot(model)
+        if hasattr(model, "n_iter_"):
+            arrays["n_iter_"] = np.asarray(model.n_iter_)
+    if not write:
+        return
+    arrays = {k.replace("/", "."): np.atleast_1d(np.asarray(v, dtype=np.float64)) for k, v in arrays.items() if np.size(v) > 0}
+
+    def sample(a, rows):
+        if a.shape[0] <= rows:
+            return a
+        return a[np.sort(np.random.default_rng(a.shape[0]).choice(a.shape[0], rows, replace=False))]
+
+    rows = DUMP_ROWS
+    out = {k: sample(a, rows) for k, a in arrays.items()}
+    while rows > 1 and sum(a.nbytes for a in out.values()) > DUMP_BYTES:
+        rows //= 2
+        out = {k: sample(a, rows) for k, a in arrays.items()}
+    os.makedirs(out_dir, exist_ok=True)
+    for k, a in out.items():
+        np.save(os.path.join(out_dir, k + ".npy"), a)
 
 
 # ------------------------------------------------------------------------------------------------
@@ -135,7 +182,7 @@ def cpu_sample(args, p_sample, repeats=1, n=None, nan_frac=None):
     best = min(times)
     what = "mbpls/mbpls.py of the reference (unmodified, check_array shim)" if use_ref else "oracle numpy/OpenBLAS port of mbpls.py"
     return dict(seconds=best, mean_seconds=sum(times) / len(times), gbs=fit_bytes(n, p, K, trips) / best / 1e9, trips=trips,
-                cores=threads, kind="reference" if use_ref else "port", p=p, n=n,
+                cores=threads, kind="reference" if use_ref else "port", p=p, n=n, model=m,
                 sample=f"{what}, NIPALS, n={n}, p={p} in 4 blocks, q={args.q}, K={K}, nan_frac={nan_frac}, "
                        f"{threads} BLAS threads of {os.cpu_count()} cpus, best of {repeats}")
 
@@ -160,6 +207,8 @@ def run_reference(args):
     for _ in range(steps):
         res = cpu_sample(args, p_sample)
         times.append(res["seconds"])
+    if args.dump_outputs:
+        dump_outputs(res["model"], args.dump_outputs)
     sec = sum(times) / len(times)
     gbs = res["gbs"] * res["seconds"] / sec
     # a second width: the fit time is linear in p (so GB/s at the sample width stands for the full width), and the NaN-mode
@@ -173,7 +222,7 @@ def run_reference(args):
         extra["nan_10pct"] = {"value": nan["gbs"], "unit": "GB/s", "seconds": nan["seconds"], "cores": nan["cores"], "kind": nan["kind"],
                               "sample": nan["sample"]}
     line = {
-        "impl": "reference", "metric": METRIC, "value": gbs, "unit": "GB/s", "n_gpus": args.gpus, "steps": steps,
+        "impl": "reference", "metric": METRIC, "value": gbs, "unit": "GB/s", "n_gpus": args.gpus, "steps": len(times),
         "warmup": warm, "ms_per_step": sec * 1e3, "higher_is_better": True, "scaling": "strong", "vs_baseline": None,
         "dtype": "f64", "data": "synthetic",
         "config": workload_config(args, note=f"bounded CPU sample: p={res['p']} features instead of {int(sum(SIZES_FULL) * args.scale)} "
@@ -181,7 +230,7 @@ def run_reference(args):
         "trips_per_component": res["trips"], "best_of_steps_s": min(times),
         "cpu_baseline": {"value": gbs, "unit": "GB/s", "cores": res["cores"], "kind": res["kind"], "sample": res["sample"]},
         "e2e": {"value": gbs, "unit": "GB/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0},
-        "gpu_launches": 0, **extra,
+        "gpu_launches": 0, "step_ms": [t * 1e3 for t in times], **extra,
     }
     print(json.dumps(line), flush=True)
 
@@ -637,6 +686,8 @@ def run_ours(args):
         log("timed fit ms", ms)
     launches = _cabi.launch_count - launches0
     clk = clocks.stop() if clocks else None
+    if args.dump_outputs:  # N > 1: rank 0's feature shard of the per-feature attributes
+        dump_outputs(model, args.dump_outputs, write=rank == 0)
     # BASELINE config 4 as written: the same fit with 10 % i.i.d. NaN holes (sparse_data=True), reported beside the headline
     variants = {}
     if args.nan_frac == 0 and not args.no_nan_variant:

@@ -2,8 +2,8 @@
 import ctypes
 import os
 import re
-
-import pytest
+import subprocess
+import sys
 
 from mbpls_b200 import _cabi
 
@@ -29,13 +29,17 @@ def test_library_exports_every_declared_symbol():
 
 
 def test_product_path_fails_loudly_without_gpu():
-    import torch
-    from mbpls_b200 import MBPLS
-    import numpy as np
-    if torch.cuda.is_available():
-        pytest.skip("GPU present")
-    with pytest.raises(_cabi.MbplsCudaError):
-        MBPLS(n_components=1).fit(np.random.rand(5, 3), np.random.rand(5))
+    # in a child process that sees no CUDA device, so that this also runs on a machine with a GPU
+    code = ("import numpy as np\n"
+            "from mbpls_b200 import MBPLS, _cabi\n"
+            "try:\n"
+            "    MBPLS(n_components=1).fit(np.random.rand(5, 3), np.random.rand(5))\n"
+            "except _cabi.MbplsCudaError:\n"
+            "    raise SystemExit(0)\n"
+            "raise SystemExit('fit did not raise MbplsCudaError without a CUDA device')\n")
+    r = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True, timeout=300, cwd=ROOT,
+                       env=dict(os.environ, CUDA_VISIBLE_DEVICES=""))
+    assert r.returncode == 0, r.stdout[-2000:] + r.stderr[-2000:]
 
 
 def test_product_never_imports_oracle():
