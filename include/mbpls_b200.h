@@ -26,7 +26,7 @@
 extern "C" {
 #endif
 
-#define MBPLS_ABI_VERSION 15
+#define MBPLS_ABI_VERSION 16
 
 /* indices into the per-fit scalar / control buffers */
 #define MBPLS_SCAL_UU 0    /* u'u of the current Y-score vector (mbpls.py:847,856,879) */
@@ -238,7 +238,17 @@ int mbpls_fused_standardize_f64(double* Xt, long ld, int n, const double* u0, co
  * Xw [nfits][p*ldw] / Yw [nfits][q*ldw] receive the standardised (then deflated) copies; scratch holds
  * mbpls_smallfit_scratch_doubles(...) doubles per fit (scratch_stride).  With preds != NULL the CTA also predicts the
  * samples test_idx[f*ld_tidx .. + test_cnt[f]) for every prefix of its model: preds[k][sample][c], k+1 components
- * (the leading blocks of P'W, :1386).  Dense data only. */
+ * (the leading blocks of P'W, :1386).  Dense data only.
+ * Resampling (permutation tests, bootstrap); every field below left zero / NULL keeps the behaviour above:
+ *   ytrain_idx  per fit, ld_idx wide, counts of train_cnt: the rows of Ysrc gathered for the fit (NULL: those of train_idx);
+ *               X row train_idx[t] is paired with Y row ytrain_idx[t] (a permuted y, a bootstrap resample)
+ *   fit_preds   held-out predictions per fit by position in its test list: fit_preds[((f*K + k)*ld_tidx + t)*q + c], k+1
+ *               components, computed like preds (one of preds and fit_preds, not both)
+ *   nslots      0: a grid of nfits CTAs, everything indexed by fit.  > 0: a grid of nslots persistent CTAs; each claims the
+ *               next fit with atomicAdd(ticket, 1) until the claims reach nfits.  Xw, Yw, scratch, stats, Wt, W, P, Ts, U, Tb
+ *               and R are then indexed by slot (the CTA), small, beta and fit_preds by fit; beta may be NULL (not written);
+ *               preds (indexed by sample) is rejected.  A fit's results do not depend on the mode or on the slot that ran it.
+ *   ticket      one int, zeroed on the launch stream by the entry point (slot mode only). */
 typedef struct mbpls_smallfit_args {
   int n_src, p, B, q, K, nfits;
   long ldx;
@@ -269,6 +279,10 @@ typedef struct mbpls_smallfit_args {
   double* preds;
   double* scratch;
   long scratch_stride;
+  const int* ytrain_idx;
+  double* fit_preds;
+  int nslots;
+  int* ticket;
 } mbpls_smallfit_args;
 int mbpls_smallfit_scratch_doubles(int p, int B, long ldw);
 int mbpls_smallfit_nipals_f64(const mbpls_smallfit_args* args_host, void* stream);

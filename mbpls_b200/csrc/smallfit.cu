@@ -13,6 +13,11 @@
 // (p_k.w_k), and beta_k = beta_{k-1} + r_k v_k' (:986-989 for every leading block at once).
 //
 // Reductions have fixed shapes (warp shuffles + fixed-order block sums), so results are bitwise reproducible.
+//
+// Slot mode (nslots > 0, permutation tests and bootstrap: 10^4 - 10^5 fits): a grid of nslots persistent CTAs, each claiming
+// the next fit from a ticket counter until none is left, so the workspace is bounded by the slots instead of the fits and a
+// slot whose fit converged early (trip counts vary a lot under a permuted PLS2 y) takes the next one.  The arithmetic of a fit
+// reads only its own inputs and workspace, so its results are bitwise the same whichever slot runs it, and in either mode.
 #include "launch.cuh"
 #include "../../include/mbpls_b200.h"
 
@@ -71,37 +76,47 @@ __device__ __forceinline__ double sf_ingest_feature(const double* __restrict__ s
   return z2;
 }
 
-__global__ void __launch_bounds__(SF_THREADS, 1) smallfit_kernel(const mbpls_smallfit_args a) {
+__shared__ int s_fit;  // slot mode: the fit thread 0 claimed for the CTA
+
+// The fit the calling CTA runs, and its workspace: the fit in per-fit mode, the CTA's slot in slot mode.  Derived again where
+// needed rather than held in registers through the component loop (the kernel has none to spare).
+__device__ __forceinline__ int sf_cur_fit(const mbpls_smallfit_args& a) { return a.nslots > 0 ? s_fit : static_cast<int>(blockIdx.x); }
+__device__ __forceinline__ size_t sf_cur_ws(const mbpls_smallfit_args& a) { return a.nslots > 0 ? blockIdx.x : sf_cur_fit(a); }
+
+// One whole fit by the calling CTA: inputs and outputs (small, beta, fit_preds) of fit sf_cur_fit, workspace sf_cur_ws.
+__device__ __forceinline__ void sf_fit(const mbpls_smallfit_args& a) {
   __shared__ double scratch[32 * 4];
   __shared__ double s_part[SF_THREADS];  // partial block scores [group][sample]
   __shared__ double s_nb[SF_MAXB], s_a[SF_MAXB], s_v[SF_MAXQ];
   __shared__ double s_sc[8];
   __shared__ int s_off[SF_MAXB + 1];
 
-  const int f = blockIdx.x;
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   const int p = a.p, B = a.B, q = a.q, K = a.K;
   const long ldw = a.ldw;
+  const int f = sf_cur_fit(a);
+  const size_t ws = sf_cur_ws(a);
   const int ntr = a.train_cnt ? a.train_cnt[f] : a.n_src;  // train_idx == NULL: every sample of the source, in order
   const int* __restrict__ tr = a.train_idx ? a.train_idx + static_cast<size_t>(f) * a.ld_idx : nullptr;
+  const int* __restrict__ ytr = a.ytrain_idx ? a.ytrain_idx + static_cast<size_t>(f) * a.ld_idx : tr;
 
-  double* Xw = a.Xw + static_cast<size_t>(f) * p * ldw;
-  double* Yw = a.Yw + static_cast<size_t>(f) * q * ldw;
-  double* stats = a.stats + static_cast<size_t>(f) * (4 * static_cast<size_t>(p) + 4 * q);
+  double* Xw = a.Xw + ws * p * ldw;
+  double* Yw = a.Yw + ws * q * ldw;
+  double* stats = a.stats + ws * (4 * static_cast<size_t>(p) + 4 * q);
   double *xmean = stats, *xvar = stats + p, *xscale = stats + 2 * static_cast<size_t>(p), *xzss = stats + 3 * static_cast<size_t>(p);
   double *ymean = stats + 4 * static_cast<size_t>(p), *yvar = ymean + q, *yscale = ymean + 2 * q, *yzss = ymean + 3 * q;
-  double* Wt = a.Wt + static_cast<size_t>(f) * K * p;
-  double* W = a.W + static_cast<size_t>(f) * K * p;
-  double* P = a.P + static_cast<size_t>(f) * K * p;
-  double* Ts = a.Ts + static_cast<size_t>(f) * K * ldw;
-  double* U = a.U + static_cast<size_t>(f) * K * ldw;
-  double* Tb = a.Tb + static_cast<size_t>(f) * B * K * ldw;
+  double* Wt = a.Wt + ws * K * p;
+  double* W = a.W + ws * K * p;
+  double* P = a.P + ws * K * p;
+  double* Ts = a.Ts + ws * K * ldw;
+  double* U = a.U + ws * K * ldw;
+  double* Tb = a.Tb + ws * B * K * ldw;
   // small: V (K*q) | A (K*B) | pssb (K*B) | tt (K) | vv (K) | diff (K) | trips (K) | varxb (B) | vary (1) | singular (1)
   double* small = a.small + static_cast<size_t>(f) * (static_cast<size_t>(K) * (q + 2 * B + 4) + B + 2);
   double *V = small, *A = V + static_cast<size_t>(K) * q, *pssb = A + static_cast<size_t>(K) * B, *ttv = pssb + static_cast<size_t>(K) * B,
          *vvv = ttv + K, *diffv = vvv + K, *tripsv = diffv + K, *varxb = tripsv + K, *vary = varxb + B, *singular = vary + 1;
   // scratch vectors: u | ts | ts_old | T (B*ldw) | w (p)
-  double* sv = a.scratch + static_cast<size_t>(f) * a.scratch_stride;
+  double* sv = a.scratch + ws * a.scratch_stride;
   double *u = sv, *ts = u + ldw, *ts_old = ts + ldw, *T = ts_old + ldw, *w = T + static_cast<size_t>(B) * ldw;
 
   for (int b = tid; b <= B; b += SF_THREADS) s_off[b] = a.block_off[b];
@@ -114,7 +129,7 @@ __global__ void __launch_bounds__(SF_THREADS, 1) smallfit_kernel(const mbpls_sma
     if (lane == 0) xzss[j] = z2;
   }
   for (int c = warp; c < q; c += SF_WARPS) {
-    const double z2 = sf_ingest_feature(a.Ysrc + static_cast<size_t>(c) * a.ldx, tr, ntr, Yw + static_cast<size_t>(c) * ldw,
+    const double z2 = sf_ingest_feature(a.Ysrc + static_cast<size_t>(c) * a.ldx, ytr, ntr, Yw + static_cast<size_t>(c) * ldw,
                                         a.standardize, ymean + c, yvar + c, yscale + c, lane);
     if (lane == 0) yzss[c] = z2;
   }
@@ -337,8 +352,8 @@ __global__ void __launch_bounds__(SF_THREADS, 1) smallfit_kernel(const mbpls_sma
   // ---- R = W (P'W)^-1 and beta = R V' (:986-989): W = concat(W_non_normal) / column norm; P'W is upper triangular for
   // NIPALS, so r_k follows by substitution over k (and the leading blocks give every prefix model).  A (near-)singular P'W --
   // more components than the data has rank -- is flagged instead: the host then applies the pseudo-inverse like the reference.
-  double* R = a.R + static_cast<size_t>(f) * K * p;
-  double* beta = a.beta + static_cast<size_t>(f) * q * p;
+  double* R = a.R + sf_cur_ws(a) * K * p;
+  double* beta = a.beta ? a.beta + static_cast<size_t>(sf_cur_fit(a)) * q * p : nullptr;
   double dmin_abs = INFINITY, dmax_abs = 0.0;
   for (int k = 0; k < K; ++k) {
     double s = 0.0;
@@ -365,7 +380,7 @@ __global__ void __launch_bounds__(SF_THREADS, 1) smallfit_kernel(const mbpls_sma
     for (int j = tid; j < p; j += SF_THREADS) R[static_cast<size_t>(k) * p + j] /= d;
     __syncthreads();
   }
-  for (int j = tid; j < p; j += SF_THREADS) {
+  for (int j = tid; beta && j < p; j += SF_THREADS) {
     for (int c = 0; c < q; ++c) {
       double acc = 0.0;
       for (int k = 0; k < K; ++k) acc = fma(R[static_cast<size_t>(k) * p + j], V[static_cast<size_t>(k) * q + c], acc);
@@ -375,10 +390,11 @@ __global__ void __launch_bounds__(SF_THREADS, 1) smallfit_kernel(const mbpls_sma
   if (tid == 0) *singular = (!(dmin_abs > 1e-10 * dmax_abs) || !isfinite(dmax_abs)) ? 1.0 : 0.0;
 
   // ---- held-out predictions for every prefix of the model (cross-validation)
-  if (!a.preds || !a.test_idx) return;
+  if ((!a.preds && !a.fit_preds) || !a.test_idx) return;
   __syncthreads();
-  const int nte = a.test_cnt[f];
-  const int* __restrict__ te = a.test_idx + static_cast<size_t>(f) * a.ld_tidx;
+  const int fit = sf_cur_fit(a);
+  const int nte = a.test_cnt[fit];
+  const int* __restrict__ te = a.test_idx + static_cast<size_t>(fit) * a.ld_tidx;
   // y_hat_k(x) = sum_{j<=k} (z . r_j) v_j, z the standardised sample; back to the Y scale (:1386)
   for (int t = 0; t < nte; ++t) {
     const int idx = te[t];
@@ -393,15 +409,32 @@ __global__ void __launch_bounds__(SF_THREADS, 1) smallfit_kernel(const mbpls_sma
       if (lane == 0) s_part[k] = s;
     }
     __syncthreads();
+    // preds[k][idx][c] (by sample) or fit_preds[f][k][t][c] (by position in the fit's test list)
+    double* dst = a.preds ? a.preds + static_cast<size_t>(idx) * q : a.fit_preds + (static_cast<size_t>(fit) * K * a.ld_tidx + t) * q;
+    const size_t kstep = static_cast<size_t>(a.preds ? a.n_src : a.ld_tidx) * q;
     for (int c = tid; c < q; c += SF_THREADS) {
       double acc = 0.0;
       for (int k = 0; k < K; ++k) {
         acc = fma(s_part[k], V[static_cast<size_t>(k) * q + c], acc);
         const double yh = a.standardize ? acc * yscale[c] + ymean[c] : acc;
-        a.preds[(static_cast<size_t>(k) * a.n_src + idx) * q + c] = yh;
+        dst[k * kstep + c] = yh;
       }
     }
     __syncthreads();
+  }
+}
+
+// Both modes go through the one inlined copy of sf_fit, so a fit compiles to the same instructions in either.
+__global__ void __launch_bounds__(SF_THREADS, 1) smallfit_kernel(const mbpls_smallfit_args a) {
+  while (true) {
+    if (a.nslots > 0) {  // thread 0 claims the next fit for the whole CTA
+      if (threadIdx.x == 0) s_fit = atomicAdd(a.ticket, 1);
+      __syncthreads();
+      if (s_fit >= a.nfits) return;
+    }
+    sf_fit(a);
+    if (a.nslots == 0) return;
+    __syncthreads();  // the slot's workspace, s_fit and the shared arrays are reused by the next fit
   }
 }
 
@@ -416,15 +449,22 @@ int mbpls_smallfit_scratch_doubles(int p, int B, long ldw) {
 
 int mbpls_smallfit_nipals_f64(const mbpls_smallfit_args* a, void* stream) {
   if (!a || !a->Xsrc || !a->Ysrc || !a->block_off || (a->train_idx && !a->train_cnt) || !a->Xw || !a->Yw || !a->stats || !a->Wt ||
-      !a->W || !a->P || !a->Ts || !a->U || !a->Tb || !a->small || !a->R || !a->beta || !a->scratch)
+      !a->W || !a->P || !a->Ts || !a->U || !a->Tb || !a->small || !a->R || (!a->beta && a->nslots == 0) || !a->scratch)
     return MBPLS_ERR_ARG;
+  if (a->nslots < 0 || (a->nslots > 0 && (!a->ticket || a->preds))) return MBPLS_ERR_ARG;  // preds: test sets may overlap
+  if ((a->ytrain_idx && !a->train_idx) || (a->fit_preds && (a->preds || !a->test_idx || !a->test_cnt))) return MBPLS_ERR_ARG;
   if (a->B < 1 || a->B > SF_MAXB || a->q < 1 || a->q > SF_MAXQ || a->K < 1 || a->K > SF_THREADS || a->p < 1 || a->nfits < 1)
     return MBPLS_ERR_SIZE;
   if (a->preds && (!a->test_idx || !a->test_cnt)) return MBPLS_ERR_ARG;
   if (!a->train_idx && (a->nfits != 1 || a->ldw < a->n_src)) return MBPLS_ERR_ARG;
   const int need = mbpls_smallfit_scratch_doubles(a->p, a->B, a->ldw);
   if (need < 0 || a->scratch_stride < need) return MBPLS_ERR_ARG;
-  smallfit_kernel<<<a->nfits, SF_THREADS, 0, static_cast<cudaStream_t>(stream)>>>(*a);
+  const cudaStream_t st = static_cast<cudaStream_t>(stream);
+  if (a->nslots > 0) {
+    const cudaError_t e = cudaMemsetAsync(a->ticket, 0, sizeof(int), st);
+    if (e != cudaSuccess) return MBPLS_CUDA_ERR(e);
+  }
+  smallfit_kernel<<<a->nslots > 0 ? a->nslots : a->nfits, SF_THREADS, 0, st>>>(*a);
   MBPLS_RETURN_LAST();
 }
 

@@ -551,18 +551,8 @@ class MBPLS(TransformerMixin, RegressorMixin, MultiOutputMixin, BaseEstimator):
                                           for b in range(B)]
             lazy["y_scaler_"] = lambda: _make_scaler(st_h[4 * p:4 * p + q], st_h[4 * p + q:4 * p + 2 * q],
                                                      st_h[4 * p + 2 * q:4 * p + 3 * q], np.full(q, n, dtype=np.int64))
-        A = np.ascontiguousarray(sm["A"].T)
-        self.A_ = A
-        if self.calc_all:  # mbpls.py:932-964 from the reduced scalars
-            tt, vv, pssb, varxb = sm["tt"], sm["vv"], sm["pssb"], sm["varxb"]
-            self.explained_var_x_ = [float(tt[k] * pssb[k].sum() / varxb.sum()) for k in range(K)]
-            self.explained_var_y_ = [float(tt[k] * vv[k] / sm["vary"]) for k in range(K)]
-            self.explained_var_xblocks_ = (tt[None, :] * pssb.T) / varxb[:, None]
-            self.A_corrected_ = np.stack([_bip_corrected(A[:, k], shard.sizes) for k in range(K)], axis=1)
-        else:
-            self.explained_var_x_, self.explained_var_y_ = [], []
-            self.explained_var_xblocks_ = np.empty((B, 0))
-            self.A_corrected_ = np.empty((B, 0))
+        for name, v in _small_attributes(sm, shard.sizes, self.calc_all).items():
+            setattr(self, name, v)
         self.W_concat_ = np.empty((p, 0))
         off = shard.block_off
         split = lambda M_: [np.ascontiguousarray(M_[:, off[b]:off[b + 1]].T) for b in range(B)]
@@ -993,6 +983,22 @@ def _make_scaler(mean, var, scale, seen) -> StandardScaler:
     sc.n_samples_seen_ = seen[0] if seen.size and np.ptp(seen) == 0 else seen
     sc.n_features_in_ = int(sc.mean_.shape[0])
     return sc
+
+
+def _small_attributes(sm: dict, sizes, calc_all: bool) -> dict:
+    """A_, and with calc_all A_corrected_ and the explained variances (mbpls.py:932-964), of one fit of the one-kernel path
+    from the reduced scalars of its `small` block (smallfit.unpack_small)."""
+    A = np.ascontiguousarray(sm["A"].T)
+    B, K = A.shape
+    if not calc_all:
+        return dict(A_=A, explained_var_x_=[], explained_var_y_=[], explained_var_xblocks_=np.empty((B, 0)),
+                    A_corrected_=np.empty((B, 0)))
+    tt, vv, pssb, varxb = sm["tt"], sm["vv"], sm["pssb"], sm["varxb"]
+    return dict(A_=A,
+                explained_var_x_=[float(tt[k] * pssb[k].sum() / varxb.sum()) for k in range(K)],
+                explained_var_y_=[float(tt[k] * vv[k] / sm["vary"]) for k in range(K)],
+                explained_var_xblocks_=(tt[None, :] * pssb.T) / varxb[:, None],
+                A_corrected_=np.stack([_bip_corrected(A[:, k], sizes) for k in range(K)], axis=1))
 
 
 def _bip_corrected(a, sizes):

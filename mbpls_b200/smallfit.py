@@ -25,7 +25,8 @@ from .engine import F64, ptr, stream_ptr
 # a fit runs in one CTA when its matrix has at most this many elements (1 MB of fp64): beyond it the single SM's L2
 # bandwidth costs more than the launches it saves
 SMALL_ELEMS = 1 << 17
-# cross-validation: all folds at once when their private copies of the training data fit this many bytes
+# cross-validation: all folds at once when their private copies of the training data fit this many bytes; permutation
+# tests and bootstrap (slot mode): the per-fit outputs of one launch
 CV_WORKSPACE_BYTES = 4 << 30
 
 
@@ -37,6 +38,30 @@ def eligible(method: str, sparse: bool, group, n: int, p: int, force) -> bool:
     if force is None and os.environ.get("MBPLS_SMALL_PATH", "1") == "0":
         return False
     return bool(force) or n * p <= SMALL_ELEMS
+
+
+def batch_eligible(estimator, ntr_max: int, p: int) -> bool:
+    """Slot-mode batches (permutation tests, bootstrap) of dense NIPALS fits: the workspace is bounded by the slots, so only
+    the size of one fit decides (small_path None: automatic, False: never, True: always)."""
+    rt = estimator._runtime()
+    force = rt["small_path"]
+    if force is False or estimator.method != 'NIPALS' or estimator.sparse_data or rt["group"] is not None:
+        return False
+    if force is None:
+        return os.environ.get("MBPLS_SMALL_PATH", "1") != "0" and ntr_max * p <= 8 * SMALL_ELEMS
+    return True
+
+
+def slot_count(device, nfits: int) -> int:
+    """Persistent CTAs of a slot-mode launch: one 1024-thread CTA per SM, no more than there are fits."""
+    return max(1, min(nfits, torch.cuda.get_device_properties(device).multi_processor_count))
+
+
+def unit_batches(n_units: int, fits_per_unit: int, bytes_per_fit: int) -> list:
+    """[u0, u1) ranges of whole units (a permutation's folds, a resample) whose per-fit outputs fit CV_WORKSPACE_BYTES each:
+    one range, i.e. one launch, unless the request is larger than that."""
+    per = max(1, CV_WORKSPACE_BYTES // max(1, fits_per_unit * bytes_per_fit))
+    return [(u, min(n_units, u + per)) for u in range(0, n_units, per)]
 
 
 def pack_source(blocks: Sequence, Y, device):
@@ -72,25 +97,36 @@ def pack_source(blocks: Sequence, Y, device):
     return H.to(device, non_blocking=True), n, sizes, p, q, ldx
 
 
+PER_FIT = ("small", "beta")  # sections indexed by fit in slot mode too; the others are indexed by slot
+
+
 @dataclass
 class Layout:
-    """Offsets (in doubles) of the per-fit result sections inside the packed output buffer."""
+    """Offsets (in doubles) of the result sections inside the packed output buffer: one entry per fit, or in slot mode
+    (nslots > 0) one per slot for every section but `small` and `beta` (no `beta` section without want_beta)."""
     nfits: int
     p: int
     q: int
     B: int
     K: int
     ldw: int
+    nslots: int = 0
+    want_beta: bool = True
 
     def __post_init__(self):
         p, q, B, K, ldw, F = self.p, self.q, self.B, self.K, self.ldw, self.nfits
         self.sizes = dict(stats=4 * p + 4 * q, Wt=K * p, W=K * p, P=K * p, Ts=K * ldw, U=K * ldw, Tb=B * K * ldw,
-                          small=K * (q + 2 * B + 4) + B + 2, R=K * p, beta=q * p)
+                          small=K * (q + 2 * B + 4) + B + 2, R=K * p, beta=q * p if self.want_beta else 0)
         self.off, o = {}, 0
         for name, sz in self.sizes.items():
             self.off[name] = o
-            o += sz * F
+            o += sz * (F if name in PER_FIT or not self.nslots else self.nslots)
         self.total = o
+
+    def section(self, buf, name):
+        """Every entry of a section, one row each."""
+        n = self.nfits if name in PER_FIT or not self.nslots else self.nslots
+        return buf[self.off[name]:self.off[name] + n * self.sizes[name]].reshape(n, self.sizes[name])
 
     def view(self, buf, name, f=0):
         sz = self.sizes[name]
@@ -100,9 +136,14 @@ class Layout:
 
 def launch(D: torch.Tensor, n_src: int, p: int, q: int, ldx: int, block_off: Sequence[int], K: int, standardize: bool,
            norm_kind: int, max_tol: float, max_iter: int, train_sets: Optional[List[np.ndarray]],
-           test_sets: Optional[List[np.ndarray]] = None):
+           test_sets: Optional[List[np.ndarray]] = None, *, y_sets: Optional[List[np.ndarray]] = None, nslots: int = 0,
+           fit_preds: bool = False, want_beta: bool = True):
     """Run ``len(train_sets)`` fits concurrently (train_sets None: one fit on all samples).  ``D`` is pack_source's buffer.
-    Returns (layout, packed device result buffer, preds device tensor or None, buffers to keep alive)."""
+    y_sets: per fit, the Y rows paired with its X rows train_sets[f] (None: the same rows).  nslots > 0: slot mode, that many
+    persistent CTAs work through the fits, workspace per slot (nslots 0: one CTA and one workspace per fit).  fit_preds: the
+    held-out predictions per fit, (nfits, K, max test size, q), instead of by sample (K, n_src, q; not in slot mode).
+    want_beta False: no beta section (slot mode only).
+    Returns (layout, packed device result buffer, predictions device tensor or None, buffers to keep alive)."""
     dev = D.device
     B = len(block_off) - 1
     boff_ptr = C.c_void_p(D.data_ptr() + 8 * (p + q) * ldx)  # the table pack_source put behind the matrix
@@ -114,30 +155,38 @@ def launch(D: torch.Tensor, n_src: int, p: int, q: int, ldx: int, block_off: Seq
         F = len(train_sets)
         ld_idx = max(len(t) for t in train_sets)
         ldw = (ld_idx + 1) // 2 * 2
-        tr = np.zeros((F, ld_idx), dtype=np.int32)
-        cnt = np.zeros(F, dtype=np.int32)
-        for f, t in enumerate(train_sets):
-            tr[f, :len(t)] = t
-            cnt[f] = len(t)
-        ints = [tr.ravel(), cnt]
+
+        def table(sets, ld):
+            idx = np.zeros((F, ld), dtype=np.int32)
+            cnt = np.zeros(F, dtype=np.int32)
+            for f, t in enumerate(sets):
+                idx[f, :len(t)] = t
+                cnt[f] = len(t)
+            return idx.ravel(), cnt
+
+        ints = list(table(train_sets, ld_idx))
         ld_t = 0
         if test_sets is not None:
             ld_t = max(1, max(len(t) for t in test_sets))
-            te = np.zeros((F, ld_t), dtype=np.int32)
-            tcnt = np.zeros(F, dtype=np.int32)
-            for f, t in enumerate(test_sets):
-                te[f, :len(t)] = t
-                tcnt[f] = len(t)
-            ints += [te.ravel(), tcnt]
+            ints += table(test_sets, ld_t)
+        if y_sets is not None:
+            ints.append(table(y_sets, ld_idx)[0])
+        if nslots:
+            ints.append(np.zeros(1, dtype=np.int32))  # the ticket counter (zeroed again on the stream by the entry point)
         packed = torch.from_numpy(np.concatenate(ints)).to(dev, non_blocking=True)  # every index table in one copy
         offs = np.cumsum([0] + [len(a) for a in ints])
         iptr = lambda i: C.c_void_p(packed.data_ptr() + 4 * int(offs[i]))
-    lay = Layout(F, p, q, B, K, ldw)
+    nt = 4 if test_sets is not None else 2  # tables before the Y rows and the ticket
+    S = nslots or F  # workspaces
+    lay = Layout(F, p, q, B, K, ldw, nslots, want_beta)
     out = torch.empty(lay.total, dtype=F64, device=dev)
-    work = torch.empty(F * (p + q) * ldw, dtype=F64, device=dev)
+    work = torch.empty(S * (p + q) * ldw, dtype=F64, device=dev)
     sstride = call("mbpls_smallfit_scratch_doubles", p, B, ldw)
-    scratch = torch.empty(F * sstride, dtype=F64, device=dev)
-    preds = torch.full((K, n_src, q), float("nan"), dtype=F64, device=dev) if test_sets is not None else None
+    scratch = torch.empty(S * sstride, dtype=F64, device=dev)
+    preds = None
+    if test_sets is not None:
+        shape = (F, K, ld_t, q) if fit_preds else (K, n_src, q)
+        preds = torch.full(shape, float("nan"), dtype=F64, device=dev)
     base = out.data_ptr()
     sec = lambda name: C.c_void_p(base + 8 * lay.off[name])
     args = _cabi.SmallFitArgs(
@@ -145,9 +194,11 @@ def launch(D: torch.Tensor, n_src: int, p: int, q: int, ldx: int, block_off: Seq
         standardize=1 if standardize else 0, norm_kind=norm_kind, max_iter=int(min(max_iter, 2**31 - 1)), max_tol=float(max_tol),
         train_idx=iptr(0), train_cnt=iptr(1), ld_idx=ld_idx,
         test_idx=iptr(2) if test_sets is not None else None, test_cnt=iptr(3) if test_sets is not None else None, ld_tidx=ld_t,
-        ldw=ldw, Xw=work.data_ptr(), Yw=work.data_ptr() + 8 * F * p * ldw, stats=sec("stats"), Wt=sec("Wt"), W=sec("W"), P=sec("P"),
-        Ts=sec("Ts"), U=sec("U"), Tb=sec("Tb"), small=sec("small"), R=sec("R"), beta=sec("beta"),
-        preds=preds.data_ptr() if preds is not None else None, scratch=scratch.data_ptr(), scratch_stride=sstride)
+        ldw=ldw, Xw=work.data_ptr(), Yw=work.data_ptr() + 8 * S * p * ldw, stats=sec("stats"), Wt=sec("Wt"), W=sec("W"), P=sec("P"),
+        Ts=sec("Ts"), U=sec("U"), Tb=sec("Tb"), small=sec("small"), R=sec("R"), beta=sec("beta") if want_beta else None,
+        preds=preds.data_ptr() if preds is not None and not fit_preds else None, scratch=scratch.data_ptr(), scratch_stride=sstride,
+        ytrain_idx=iptr(nt) if y_sets is not None else None, fit_preds=preds.data_ptr() if fit_preds and preds is not None else None,
+        nslots=int(nslots), ticket=iptr(len(ints) - 1) if nslots else None)
     call("mbpls_smallfit_nipals_f64", C.byref(args), stream_ptr(dev))
     return lay, out, preds, (packed, work, scratch)
 
