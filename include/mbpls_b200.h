@@ -26,7 +26,7 @@
 extern "C" {
 #endif
 
-#define MBPLS_ABI_VERSION 16
+#define MBPLS_ABI_VERSION 17
 
 /* indices into the per-fit scalar / control buffers */
 #define MBPLS_SCAL_UU 0    /* u'u of the current Y-score vector (mbpls.py:847,856,879) */
@@ -238,7 +238,7 @@ int mbpls_fused_standardize_f64(double* Xt, long ld, int n, const double* u0, co
  * Xw [nfits][p*ldw] / Yw [nfits][q*ldw] receive the standardised (then deflated) copies; scratch holds
  * mbpls_smallfit_scratch_doubles(...) doubles per fit (scratch_stride).  With preds != NULL the CTA also predicts the
  * samples test_idx[f*ld_tidx .. + test_cnt[f]) for every prefix of its model: preds[k][sample][c], k+1 components
- * (the leading blocks of P'W, :1386).  Dense data only.
+ * (the leading blocks of P'W, :1386).
  * Resampling (permutation tests, bootstrap); every field below left zero / NULL keeps the behaviour above:
  *   ytrain_idx  per fit, ld_idx wide, counts of train_cnt: the rows of Ysrc gathered for the fit (NULL: those of train_idx);
  *               X row train_idx[t] is paired with Y row ytrain_idx[t] (a permuted y, a bootstrap resample)
@@ -248,7 +248,15 @@ int mbpls_fused_standardize_f64(double* Xt, long ld, int n, const double* u0, co
  *               next fit with atomicAdd(ticket, 1) until the claims reach nfits.  Xw, Yw, scratch, stats, Wt, W, P, Ts, U, Tb
  *               and R are then indexed by slot (the CTA), small, beta and fit_preds by fit; beta may be NULL (not written);
  *               preds (indexed by sample) is rejected.  A fit's results do not depend on the mode or on the slot that ran it.
- *   ticket      one int, zeroed on the launch stream by the entry point (slot mode only). */
+ *   ticket      one int, zeroed on the launch stream by the entry point (slot mode only).
+ *   nanmode     1: the NaN-mode fit of sparse_data=True (mbpls.py:832-930), K <= 64.  NaN stays NaN in Xw / Yw and counts as
+ *               zero in every numerator; features, Y columns and samples with a hole on the fit's rows divide by masked sums
+ *               (:848-852, :867-872, :890-897, :903, :923-925); the Y scores start from the first Y column without a hole.
+ *               P'W is not triangular then: R = W (P'W)^-1 and every prefix model come from Gauss-Jordan elimination of
+ *               each leading block; preds / fit_preds read NaN as zero after scaling (:1379-1384).  singular = 1 also
+ *               flags a fit with no fully observed Y column (the reference draws np.random.rand) or with a feature or Y
+ *               column that has no observed value on its rows: refit it through the streaming kernels.  scratch_stride >=
+ *               mbpls_smallfit_nan_scratch_doubles(p, q, B, K, ldw). */
 typedef struct mbpls_smallfit_args {
   int n_src, p, B, q, K, nfits;
   long ldx;
@@ -283,8 +291,10 @@ typedef struct mbpls_smallfit_args {
   double* fit_preds;
   int nslots;
   int* ticket;
+  int nanmode;
 } mbpls_smallfit_args;
 int mbpls_smallfit_scratch_doubles(int p, int B, long ldw);
+int mbpls_smallfit_nan_scratch_doubles(int p, int q, int B, int K, long ldw);
 int mbpls_smallfit_nipals_f64(const mbpls_smallfit_args* args_host, void* stream);
 
 /* ---- NaN bit matrix and the masked denominators derived from it (csrc/nanmask.cu; mbpls.py:848-852, :867-872, :923-925)

@@ -11,7 +11,7 @@ import os
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "lib", "libmbpls_b200.so")
 
-ABI_VERSION = 16
+ABI_VERSION = 17
 
 # indices shared with the header
 SCAL_UU, SCAL_DIFF, SCAL_TT, SCAL_VV, SCAL_COUNT = 0, 1, 2, 3, 8
@@ -55,7 +55,7 @@ class SmallFitArgs(C.Structure):
         ("ldw", _l),
         ("Xw", _p), ("Yw", _p), ("stats", _p), ("Wt", _p), ("W", _p), ("P", _p), ("Ts", _p), ("U", _p), ("Tb", _p),
         ("small", _p), ("R", _p), ("beta", _p), ("preds", _p), ("scratch", _p), ("scratch_stride", _l),
-        ("ytrain_idx", _p), ("fit_preds", _p), ("nslots", _i), ("ticket", _p),
+        ("ytrain_idx", _p), ("fit_preds", _p), ("nslots", _i), ("ticket", _p), ("nanmode", _i),
     ]
 
 
@@ -96,6 +96,7 @@ SIGNATURES = {
     "mbpls_nipals_xchg_epilogue_f64": [C.POINTER(XchgArgs), _i, _p],
     "mbpls_nipals_record_component_f64": [C.POINTER(RecordArgs), _p],
     "mbpls_smallfit_scratch_doubles": [_i, _i, _l],
+    "mbpls_smallfit_nan_scratch_doubles": [_i, _i, _i, _i, _l],
     "mbpls_smallfit_nipals_f64": [C.POINTER(SmallFitArgs), _p],
     "mbpls_loadings_deflate_f64": [_p, _l, _i, _i, _p, _p, _p, _p, _p, _p, _i, _i, _p],
     "mbpls_fused_workers_per_sm_pair": [_l],
@@ -137,7 +138,7 @@ SIGNATURES = {
 }
 
 # functions whose int return value is a plain number, not a status
-_PLAIN = {"mbpls_abi_version", "mbpls_smallfit_scratch_doubles", "mbpls_fused_workers_per_sm_pair", "mbpls_fused_total_workers", "mbpls_fused_uses_clusters", "mbpls_nan_bitmask_ldw", "mbpls_xtu_feats_per_cta", "mbpls_xtu_num_ctas", "mbpls_gram_num_chunks",
+_PLAIN = {"mbpls_abi_version", "mbpls_smallfit_scratch_doubles", "mbpls_smallfit_nan_scratch_doubles", "mbpls_fused_workers_per_sm_pair", "mbpls_fused_total_workers", "mbpls_fused_uses_clusters", "mbpls_nan_bitmask_ldw", "mbpls_xtu_feats_per_cta", "mbpls_xtu_num_ctas", "mbpls_gram_num_chunks",
           "mbpls_xw_ctas_per_sm", "mbpls_crossprod_splits", "mbpls_crossprod_splits_syrk", "mbpls_xt_multi_chunks"}
 
 

@@ -13,8 +13,9 @@ The result equals ``cross_val_predict(clone(estimator), X, y, cv=cv)`` (tests/te
 
 Validation of a fitted model's reported quantities: ``permutation_test_score`` (does the model predict better than chance?
 the cross-validation re-run on permutations of ``y``) and ``bootstrap`` (how stable are ``A_`` / ``beta_``? refits on
-resamples of the rows).  Both need 10^3 - 10^5 fits; for dense NIPALS they all run in one slot-mode launch of
-``smallfit_kernel`` (persistent CTAs that claim fit after fit, X rows paired with permuted / resampled Y rows on the device).
+resamples of the rows).  Both need 10^3 - 10^5 fits; for NIPALS, dense or with missing values (``sparse_data=True``), they
+all run in one slot-mode launch of ``smallfit_kernel`` (persistent CTAs that claim fit after fit, X rows paired with permuted /
+resampled Y rows on the device).
 """
 from __future__ import annotations
 
@@ -117,11 +118,23 @@ def _sources(X, y):
     return blocks, Ysrc, y1d, int(Ysrc.shape[0]), int(Ysrc.shape[1]), [int(b.shape[1]) for b in blocks]
 
 
-def _require_finite(arrays):
+def _require_finite(arrays, allow_nan: bool = False):
+    """check_array's finiteness test (mbpls.py:310): NaN is accepted with sparse_data=True, +-inf never (as MBPLS.fit)."""
     for a in arrays:
+        if allow_nan:
+            bad = bool(torch.isinf(a).any()) if isinstance(a, torch.Tensor) else bool(np.isinf(a).any())
+            if bad:
+                raise ValueError("Input contains infinity or a value too large for dtype('float64').")
+            continue
         ok = bool(torch.isfinite(a).all()) if isinstance(a, torch.Tensor) else bool(np.isfinite(a).all())
         if not ok:
             raise ValueError("Input contains NaN or infinity.")
+
+
+def _nan_eligible(blocks, Ysrc, x_rows, y_rows) -> np.ndarray:
+    """smallfit.nan_fits_eligible on the source arrays: per fit, True if the NaN-mode batch can run it."""
+    x_obs = np.hstack([SF.observed(b) for b in blocks])
+    return SF.nan_fits_eligible(x_obs, SF.observed(Ysrc), x_rows, y_rows)
 
 
 def _upload(blocks, Ysrc, n, q, shard, device):
@@ -133,14 +146,16 @@ def _upload(blocks, Ysrc, n, q, shard, device):
 
 
 def _batched_small_cv(estimator, blocks, Ysrc, n, q, sizes, shard, K, ks, folds, device):
-    """All folds of a dense NIPALS cross-validation in ONE kernel launch (csrc/smallfit.cu): one CTA per fold gathers its
-    training samples from the shared source, fits K components with the loop on the device, and predicts its held-out samples
-    for every prefix 1..K of the model.  Returns {k: (n, q) array}, or None when the problem is not eligible (-> fold loop)."""
-    from . import smallfit as SF
+    """All folds of a NIPALS cross-validation in ONE kernel launch (csrc/smallfit.cu): one CTA per fold gathers its training
+    samples from the shared source, fits K components with the loop on the device, and predicts its held-out samples for
+    every prefix 1..K of the model.  sparse_data=True runs the NaN-mode fit (any method: MBPLS.fit fits NIPALS then too).
+    Returns {k: (n, q) array}, or None when the problem is not eligible, a fold's training rows are not
+    (smallfit.nan_fits_eligible) or a fold comes back flagged (-> fold loop)."""
     rt = estimator._runtime()
     p = sum(sizes)
     force = rt["small_path"]
-    if force is False or estimator.method != 'NIPALS' or estimator.sparse_data or not folds:
+    sparse = bool(estimator.sparse_data)
+    if force is False or (estimator.method != 'NIPALS' and not sparse) or not folds:
         return None
     ntr_max = max(len(tr) for tr, _ in folds)
     if force is None:
@@ -151,15 +166,14 @@ def _batched_small_cv(estimator, blocks, Ysrc, n, q, sizes, shard, K, ks, folds,
             return None
     from .mbpls import _check_limits
     _check_limits(K, q, len(sizes))
-    for a in blocks + [Ysrc]:
-        ok = bool(torch.isfinite(a).all()) if isinstance(a, torch.Tensor) else bool(np.isfinite(a).all())
-        if not ok:
-            raise ValueError("Input contains NaN or infinity.")
+    _require_finite(blocks + [Ysrc], allow_nan=sparse)
+    if sparse and not _nan_eligible(blocks, Ysrc, [tr for tr, _ in folds], [tr for tr, _ in folds]).all():
+        return None
     D, n, sizes, p, q, ldx = SF.pack_source(blocks, Ysrc, device)
     lay, out, preds_d, keep = SF.launch(D, n, p, q, ldx, shard.block_off, K, bool(estimator.standardize),
                                         E.norm_kind_of(estimator.nipals_convergence_norm), estimator.max_tol, rt["max_iter"],
                                         [np.asarray(tr, dtype=np.int32) for tr, _ in folds],
-                                        [np.asarray(te, dtype=np.int32) for _, te in folds])
+                                        [np.asarray(te, dtype=np.int32) for _, te in folds], nanmode=sparse)
     sm_all = E.to_host(out[lay.off["small"]:lay.off["small"] + lay.sizes["small"] * len(folds)]).reshape(len(folds), -1)
     if np.any(sm_all[:, -1] != 0.0):  # some fold has more components than rank: the fold loop applies the pseudo-inverse
         return None
@@ -286,8 +300,10 @@ def permutation_test_score(estimator: MBPLS, X, y, cv=5, n_permutations: int = 1
     call to call needs a fixed ``random_state``.  ``scoring``: None (the estimator's ``score``, r2), "r2",
     "explained_variance", "neg_mean_squared_error", "neg_root_mean_squared_error" or "neg_mean_absolute_error".
 
-    Dense NIPALS problems small enough for one CTA run every fit of every permutation in one kernel launch; other methods,
-    ``sparse_data=True`` or larger problems refit through ``MBPLS.fit``.
+    NIPALS problems small enough for one CTA, dense or with ``sparse_data=True``, run every fit of every permutation in one
+    kernel launch; other methods and larger problems refit through ``MBPLS.fit``, and so do the fits the batch cannot run
+    (more components than rank; with missing values, training rows that leave a feature or Y column unobserved or no Y column
+    fully observed).
     """
     _check_scoring(scoring)
     rt = estimator._runtime()
@@ -310,7 +326,7 @@ def permutation_test_score(estimator: MBPLS, X, y, cv=5, n_permutations: int = 1
         redo = fits
         if SF.batch_eligible(estimator, max(len(tr) for tr, _ in folds), sum(sizes)):
             redo = _permutation_batches(estimator, blocks, Ysrc, n, q, shard, K, kk, folds, perms, preds, device)
-        if redo:  # every fit (generic path), or the fits flagged singular, one by one through MBPLS.fit
+        if redo:  # every fit (generic path), or the fits the batch flagged or could not run, one by one through MBPLS.fit
             Xraw, Yraw = _upload(blocks, Ysrc, n, q, shard, device)
             todo = [(folds[i][0], perms[r][folds[i][0]], folds[i][1]) for r, i in redo]
             for (r, i), pred in zip(redo, _fold_predictions(estimator, Xraw, Yraw, shard, q, K, kk, todo, device)):
@@ -333,19 +349,23 @@ def permutation_test_score(estimator: MBPLS, X, y, cv=5, n_permutations: int = 1
 def _permutation_batches(estimator, blocks, Ysrc, n, q, shard, K, kk, folds, perms, preds, device) -> list:
     """Every (permutation, fold) fit in slot-mode launches of smallfit_kernel (one unless the per-fit outputs exceed
     CV_WORKSPACE_BYTES): fit (r, i) gathers X rows tr_i and Y rows pi_r[tr_i] and predicts X rows te_i for every prefix
-    model.  Fills preds; returns the (permutation, fold) pairs of the fits flagged singular (more components than rank),
-    which the caller refits."""
+    model.  Fills preds; returns the (permutation, fold) pairs of the fits flagged singular (more components than rank) or,
+    with sparse_data=True, not eligible (smallfit.nan_fits_eligible) or flagged by the kernel, which the caller refits."""
     from .mbpls import _check_limits
     rt = estimator._runtime()
+    sparse = bool(estimator.sparse_data)
     _check_limits(K, q, len(shard.sizes))
-    _require_finite(blocks + [Ysrc])
-    D, n, sizes, p, q, ldx = SF.pack_source(blocks, Ysrc, device)
+    _require_finite(blocks + [Ysrc], allow_nan=sparse)
     R, nf = perms.shape[0], len(folds)
+    redo = set()
+    if sparse:
+        ok = _nan_eligible(blocks, Ysrc, [tr for _ in range(R) for tr, _ in folds], [perms[r][tr] for r in range(R) for tr, _ in folds])
+        redo.update(divmod(int(f), nf) for f in np.flatnonzero(~ok))
+    D, n, sizes, p, q, ldx = SF.pack_source(blocks, Ysrc, device)
     B = len(sizes)
     ld_t = preds.shape[3]
     kidx = [k - 1 for k in kk]
     small_sz = K * (q + 2 * B + 4) + B + 2
-    singular = []
     for r0, r1 in SF.unit_batches(R, nf, 8 * (small_sz + K * ld_t * q)):
         F = (r1 - r0) * nf
         lay, out, fp, keep = SF.launch(
@@ -354,12 +374,12 @@ def _permutation_batches(estimator, blocks, Ysrc, n, q, shard, K, kk, folds, per
             [np.asarray(tr, dtype=np.int32) for _ in range(r0, r1) for tr, _ in folds],
             [np.asarray(te, dtype=np.int32) for _ in range(r0, r1) for _, te in folds],
             y_sets=[perms[r][tr].astype(np.int32) for r in range(r0, r1) for tr, _ in folds],
-            nslots=SF.slot_count(device, F), fit_preds=True, want_beta=False)
+            nslots=SF.slot_count(device, F), fit_preds=True, want_beta=False, nanmode=sparse)
         flags = E.to_host(lay.section(out, "small")[:, -1])
         host = E.to_host(fp)                                        # F x K x ld_t x q
         preds[r0:r1] = host[:, kidx].reshape(r1 - r0, nf, len(kk), ld_t, q)
-        singular += [divmod(r0 * nf + int(f), nf) for f in np.nonzero(flags != 0.0)[0]]
-    return singular
+        redo.update(divmod(r0 * nf + int(f), nf) for f in np.nonzero(flags != 0.0)[0])
+    return sorted(redo)
 
 
 def bootstrap(estimator: MBPLS, X, y, n_resamples: int = 100, random_state=0) -> dict:
@@ -372,8 +392,9 @@ def bootstrap(estimator: MBPLS, X, y, n_resamples: int = 100, random_state=0) ->
     (R x B x K), ``explained_var_x_`` / ``explained_var_y_`` (R x K) and ``explained_var_xblocks_`` (R x B x K).  Entry r is
     the attribute of ``clone(estimator).fit([x[idx] for x in X], y[idx])``.
 
-    Dense NIPALS problems small enough for one CTA fit every resample in one kernel launch; other methods,
-    ``sparse_data=True``, larger problems and resamples with more components than rank refit through ``MBPLS.fit``.
+    NIPALS problems small enough for one CTA, dense or with ``sparse_data=True``, fit every resample in one kernel launch;
+    other methods, larger problems and the resamples the batch cannot run (more components than rank; with missing values,
+    rows that leave a feature or Y column unobserved or no Y column fully observed) refit through ``MBPLS.fit``.
     """
     from .mbpls import _check_limits, _small_attributes
     rt = estimator._runtime()
@@ -387,22 +408,24 @@ def bootstrap(estimator: MBPLS, X, y, n_resamples: int = 100, random_state=0) ->
         (["A_corrected_", "explained_var_x_", "explained_var_y_", "explained_var_xblocks_"] if estimator.calc_all else [])
     res = {name: [None] * R for name in names}
     redo = list(range(R))
+    sparse = bool(estimator.sparse_data)
     with torch.cuda.device(device):
         shard = E.ShardMap.build(sizes, 0, 1)
         if SF.batch_eligible(estimator, n, p):
             _check_limits(K, q, B)
-            _require_finite(blocks + [Ysrc])
+            _require_finite(blocks + [Ysrc], allow_nan=sparse)
+            ok = _nan_eligible(blocks, Ysrc, idx, idx) if sparse else np.ones(R, dtype=bool)
             D, n, sizes, p, q, ldx = SF.pack_source(blocks, Ysrc, device)
             redo = []
             for r0, r1 in SF.unit_batches(R, 1, 8 * (K * (q + 2 * B + 4) + B + 2 + q * p)):
                 lay, out, _, keep = SF.launch(
                     D, n, p, q, ldx, shard.block_off, K, bool(estimator.standardize),
                     E.norm_kind_of(estimator.nipals_convergence_norm), estimator.max_tol, rt["max_iter"],
-                    [idx[r].astype(np.int32) for r in range(r0, r1)], nslots=SF.slot_count(device, r1 - r0))
+                    [idx[r].astype(np.int32) for r in range(r0, r1)], nslots=SF.slot_count(device, r1 - r0), nanmode=sparse)
                 small, beta = E.to_host(lay.section(out, "small")), E.to_host(lay.section(out, "beta"))
                 for r in range(r0, r1):
                     sm = SF.unpack_small(small[r - r0], K, q, B)
-                    if sm["singular"]:  # R = W pinv(P'W) like the reference: refit below
+                    if sm["singular"] or not ok[r]:  # R = W pinv(P'W) like the reference, or a NaN fit the batch cannot run
                         redo.append(r)
                         continue
                     attrs = _small_attributes(sm, sizes, estimator.calc_all)

@@ -1,4 +1,5 @@
-"""Whole dense NIPALS fits in one kernel launch (csrc/smallfit.cu): the launch-latency regime of the reference.
+"""Whole NIPALS fits in one kernel launch (csrc/smallfit.cu): the launch-latency regime of the reference.  Dense fits, and for
+cross-validation, permutation tests and bootstrap also fits with missing values (sparse_data=True, nanmode).
 
 The reference's README quickstart (README.rst:82-95) and the leave-one-out loops of its notebooks
 (``cross_val_predict(MBPLS(n_components=k), X, y, cv=len(X))``, examples/real_world_applications/*.ipynb) fit matrices of
@@ -41,15 +42,41 @@ def eligible(method: str, sparse: bool, group, n: int, p: int, force) -> bool:
 
 
 def batch_eligible(estimator, ntr_max: int, p: int) -> bool:
-    """Slot-mode batches (permutation tests, bootstrap) of dense NIPALS fits: the workspace is bounded by the slots, so only
-    the size of one fit decides (small_path None: automatic, False: never, True: always)."""
+    """Slot-mode batches (permutation tests, bootstrap) of NIPALS fits, dense or NaN mode (sparse_data=True fits NIPALS
+    whatever the method, as MBPLS.fit does): the workspace is bounded by the slots, so only the size of one fit decides
+    (small_path None: automatic, False: never, True: always)."""
     rt = estimator._runtime()
     force = rt["small_path"]
-    if force is False or estimator.method != 'NIPALS' or estimator.sparse_data or rt["group"] is not None:
+    if force is False or (estimator.method != 'NIPALS' and not estimator.sparse_data) or rt["group"] is not None:
         return False
     if force is None:
         return os.environ.get("MBPLS_SMALL_PATH", "1") != "0" and ntr_max * p <= 8 * SMALL_ELEMS
     return True
+
+
+def nan_fits_eligible(x_obs: np.ndarray, y_obs: np.ndarray, x_rows: Sequence, y_rows: Sequence) -> np.ndarray:
+    """Per fit, whether the NaN-mode batch runs it (True) or it goes to MBPLS.fit (False).
+
+    x_obs (n, p) / y_obs (n, q): True where the source holds a value (not NaN); x_rows[f] / y_rows[f]: the X rows of fit f and
+    the Y rows paired with them (repeats allowed).  A fit needs an observed value of every feature and every Y column on its
+    rows, and a Y column observed on all of its Y rows to start the Y scores from (mbpls.py:832-836; without one the reference
+    draws np.random.rand)."""
+    def counts(obs, rows):  # (fits, columns): observed values on each fit's rows, with multiplicity
+        n = obs.shape[0]
+        lens = np.fromiter((len(r) for r in rows), dtype=np.int64, count=len(rows))
+        flat = np.concatenate([np.asarray(r, dtype=np.int64) for r in rows]) if len(rows) else np.zeros(0, np.int64)
+        mult = np.bincount(np.repeat(np.arange(len(rows)), lens) * n + flat, minlength=len(rows) * n).reshape(len(rows), n)
+        return mult.astype(np.float64) @ obs.astype(np.float64), lens  # exact counts, through BLAS
+    xc, _ = counts(np.asarray(x_obs, dtype=bool), x_rows)
+    yc, ylen = counts(np.asarray(y_obs, dtype=bool), y_rows)
+    return (xc > 0).all(axis=1) & (yc > 0).all(axis=1) & (yc == ylen[:, None]).any(axis=1)
+
+
+def observed(a) -> np.ndarray:
+    """(n, m) host mask of the entries of a source array (numpy or torch) that are not NaN."""
+    if isinstance(a, torch.Tensor):
+        return (~torch.isnan(a)).cpu().numpy()
+    return ~np.isnan(np.asarray(a, dtype=np.float64))
 
 
 def slot_count(device, nfits: int) -> int:
@@ -137,12 +164,13 @@ class Layout:
 def launch(D: torch.Tensor, n_src: int, p: int, q: int, ldx: int, block_off: Sequence[int], K: int, standardize: bool,
            norm_kind: int, max_tol: float, max_iter: int, train_sets: Optional[List[np.ndarray]],
            test_sets: Optional[List[np.ndarray]] = None, *, y_sets: Optional[List[np.ndarray]] = None, nslots: int = 0,
-           fit_preds: bool = False, want_beta: bool = True):
+           fit_preds: bool = False, want_beta: bool = True, nanmode: bool = False):
     """Run ``len(train_sets)`` fits concurrently (train_sets None: one fit on all samples).  ``D`` is pack_source's buffer.
     y_sets: per fit, the Y rows paired with its X rows train_sets[f] (None: the same rows).  nslots > 0: slot mode, that many
     persistent CTAs work through the fits, workspace per slot (nslots 0: one CTA and one workspace per fit).  fit_preds: the
     held-out predictions per fit, (nfits, K, max test size, q), instead of by sample (K, n_src, q; not in slot mode).
-    want_beta False: no beta section (slot mode only).
+    want_beta False: no beta section (slot mode only).  nanmode: the NaN-mode fit of sparse_data=True (K <= 64); a fit the
+    kernel cannot run (see nan_fits_eligible) comes back flagged like a singular one.
     Returns (layout, packed device result buffer, predictions device tensor or None, buffers to keep alive)."""
     dev = D.device
     B = len(block_off) - 1
@@ -181,7 +209,8 @@ def launch(D: torch.Tensor, n_src: int, p: int, q: int, ldx: int, block_off: Seq
     lay = Layout(F, p, q, B, K, ldw, nslots, want_beta)
     out = torch.empty(lay.total, dtype=F64, device=dev)
     work = torch.empty(S * (p + q) * ldw, dtype=F64, device=dev)
-    sstride = call("mbpls_smallfit_scratch_doubles", p, B, ldw)
+    sstride = call("mbpls_smallfit_nan_scratch_doubles", p, q, B, K, ldw) if nanmode else \
+        call("mbpls_smallfit_scratch_doubles", p, B, ldw)
     scratch = torch.empty(S * sstride, dtype=F64, device=dev)
     preds = None
     if test_sets is not None:
@@ -198,7 +227,7 @@ def launch(D: torch.Tensor, n_src: int, p: int, q: int, ldx: int, block_off: Seq
         Ts=sec("Ts"), U=sec("U"), Tb=sec("Tb"), small=sec("small"), R=sec("R"), beta=sec("beta") if want_beta else None,
         preds=preds.data_ptr() if preds is not None and not fit_preds else None, scratch=scratch.data_ptr(), scratch_stride=sstride,
         ytrain_idx=iptr(nt) if y_sets is not None else None, fit_preds=preds.data_ptr() if fit_preds and preds is not None else None,
-        nslots=int(nslots), ticket=iptr(len(ints) - 1) if nslots else None)
+        nslots=int(nslots), ticket=iptr(len(ints) - 1) if nslots else None, nanmode=1 if nanmode else 0)
     call("mbpls_smallfit_nipals_f64", C.byref(args), stream_ptr(dev))
     return lay, out, preds, (packed, work, scratch)
 
