@@ -13,8 +13,8 @@
  *  - All matrices are float64 and FEATURE-MAJOR: a p x ld array with one feature (one column of the
  *    reference's n x p matrix) per row, ld >= n, ld % 16 == 0, padding [n, ld) zero.  Result matrices
  *    are COMPONENT-MAJOR (K x p or K x ld).  n-vectors have at least ld elements.
- *  - `stream` is a cudaStream_t passed as void*.  Functions never allocate, never synchronise and keep
- *    no global state; they return 0, a negative MBPLS_ERR_* code for bad arguments, or
+ *  - `stream` is a cudaStream_t passed as void*.  Functions never allocate, never synchronise (unless their
+ *    doc says so) and keep no global state; they return 0, a negative MBPLS_ERR_* code for bad arguments, or
  *    1000 + cudaError_t for a launch failure.
  *  - `done` arguments point at the int ctrl[MBPLS_CTRL_DONE] of a NIPALS component; when it is
  *    non-zero the kernel returns immediately (lets the host enqueue trips in batches).
@@ -26,7 +26,7 @@
 extern "C" {
 #endif
 
-#define MBPLS_ABI_VERSION 17
+#define MBPLS_ABI_VERSION 18
 
 /* indices into the per-fit scalar / control buffers */
 #define MBPLS_SCAL_UU 0    /* u'u of the current Y-score vector (mbpls.py:847,856,879) */
@@ -256,7 +256,14 @@ int mbpls_fused_standardize_f64(double* Xt, long ld, int n, const double* u0, co
  *               each leading block; preds / fit_preds read NaN as zero after scaling (:1379-1384).  singular = 1 also
  *               flags a fit with no fully observed Y column (the reference draws np.random.rand) or with a feature or Y
  *               column that has no observed value on its rows: refit it through the streaming kernels.  scratch_stride >=
- *               mbpls_smallfit_nan_scratch_doubles(p, q, B, K, ldw). */
+ *               mbpls_smallfit_nan_scratch_doubles(p, q, B, K, ldw).
+ * Block permutation tests; NULL perm_rows and fit_perm keep the behaviour above:
+ *   perm_rows   n_perm row permutations of the source, n_src ints each (entries in [0, n_src))
+ *   fit_perm    two ints per fit, (r, b): r = -1 permutes nothing; r >= 0 makes every read of source row i for a feature of
+ *               block b, in the training gather and in the held-out predictions, read row perm_rows[r*n_src + i] instead.
+ *               Y rows and the features of other blocks are untouched.  Requires train_idx; an r outside [-1, n_perm) or a
+ *               b outside [0, B) is MBPLS_ERR_ARG (the entry point reads the pairs back, one stream synchronisation).  In NaN
+ *               mode the holes of block b move with its rows, as the census is taken on the fit's gathered copy. */
 typedef struct mbpls_smallfit_args {
   int n_src, p, B, q, K, nfits;
   long ldx;
@@ -292,6 +299,9 @@ typedef struct mbpls_smallfit_args {
   int nslots;
   int* ticket;
   int nanmode;
+  const int* perm_rows;
+  int n_perm;
+  const int* fit_perm;
 } mbpls_smallfit_args;
 int mbpls_smallfit_scratch_doubles(int p, int B, long ldw);
 int mbpls_smallfit_nan_scratch_doubles(int p, int q, int B, int K, long ldw);

@@ -11,7 +11,7 @@ import os
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "lib", "libmbpls_b200.so")
 
-ABI_VERSION = 17
+ABI_VERSION = 18
 
 # indices shared with the header
 SCAL_UU, SCAL_DIFF, SCAL_TT, SCAL_VV, SCAL_COUNT = 0, 1, 2, 3, 8
@@ -56,6 +56,7 @@ class SmallFitArgs(C.Structure):
         ("Xw", _p), ("Yw", _p), ("stats", _p), ("Wt", _p), ("W", _p), ("P", _p), ("Ts", _p), ("U", _p), ("Tb", _p),
         ("small", _p), ("R", _p), ("beta", _p), ("preds", _p), ("scratch", _p), ("scratch_stride", _l),
         ("ytrain_idx", _p), ("fit_preds", _p), ("nslots", _i), ("ticket", _p), ("nanmode", _i),
+        ("perm_rows", _p), ("n_perm", _i), ("fit_perm", _p),
     ]
 
 

@@ -19,6 +19,10 @@
 // the next fit from a ticket counter until none is left, so the workspace is bounded by the slots instead of the fits and a
 // slot whose fit converged early (trip counts vary a lot under a permuted PLS2 y) takes the next one.  The arithmetic of a fit
 // reads only its own inputs and workspace, so its results are bitwise the same whichever slot runs it, and in either mode.
+//
+// Block permutation tests (perm_rows / fit_perm): a fit may read the features of one block from permuted source rows, in its
+// training gather and in its held-out predictions; Y and the other blocks keep their rows.
+#include <vector>
 #include "launch.cuh"
 #include "../../include/mbpls_b200.h"
 
@@ -39,29 +43,35 @@ __device__ __forceinline__ double sf_scale_from(double cnt, double mean, double 
 }
 
 // gather the training samples of one source feature, standardise, store; returns sum of squares of what was stored.
+// rmap != NULL (a block-permuted fit, the feature in the permuted block): training sample t reads source row rmap[tr[t]].
 // NANMODE: the nan-aware StandardScaler of csrc/ingest.cu (statistics over the observed values, NaN stored as NaN, nansum of
 // z^2) and the observed count in *cnt_out.
 template <bool NANMODE>
-__device__ __forceinline__ double sf_ingest_feature(const double* __restrict__ src, const int* __restrict__ tr, int ntr,
-                                                     double* __restrict__ dst, int standardize, double* mean_out,
-                                                     double* var_out, double* scale_out, double* cnt_out, int lane) {
+__device__ __forceinline__ double sf_ingest_feature(const double* __restrict__ src, const int* __restrict__ tr,
+                                                     const int* __restrict__ rmap, int ntr, double* __restrict__ dst,
+                                                     int standardize, double* mean_out, double* var_out, double* scale_out,
+                                                     double* cnt_out, int lane) {
+  const auto at = [&](int t) {
+    const int i = tr ? tr[t] : t;
+    return src[rmap ? rmap[i] : i];
+  };
   double mean = 0.0, var = 0.0, scale = 1.0, cnt = ntr;
   if constexpr (NANMODE) {
     double o = 0.0;
-    for (int t = lane; t < ntr; t += 32) o += isnan(src[tr ? tr[t] : t]) ? 0.0 : 1.0;
+    for (int t = lane; t < ntr; t += 32) o += isnan(at(t)) ? 0.0 : 1.0;
     cnt = warp_sum(o);
   }
   if (standardize) {
     double s = 0.0;
     for (int t = lane; t < ntr; t += 32) {
-      const double x = src[tr ? tr[t] : t];
+      const double x = at(t);
       if (!NANMODE || !isnan(x)) s += x;
     }
     s = warp_sum(s);
     mean = NANMODE ? s / cnt : s / ntr;
     double c = 0.0, ss = 0.0;
     for (int t = lane; t < ntr; t += 32) {
-      const double d = src[tr ? tr[t] : t] - mean;
+      const double d = at(t) - mean;
       if (!NANMODE || !isnan(d)) {
         c += d;
         ss += d * d;
@@ -73,7 +83,7 @@ __device__ __forceinline__ double sf_ingest_feature(const double* __restrict__ s
   }
   double z2 = 0.0;
   for (int t = lane; t < ntr; t += 32) {
-    double z = src[tr ? tr[t] : t];
+    double z = at(t);
     if (standardize) {
       z = z - mean;
       z = z / scale;
@@ -95,6 +105,7 @@ __shared__ int s_fit;   // slot mode: the fit thread 0 claimed for the CTA
 __shared__ int s_ycol;  // NaN mode: the Y column the Y scores start from (mbpls.py:832-836)
 __shared__ double s_cn[SF_MAXK], s_fac[SF_MAXK];  // NaN mode: |w~_k|; Gauss-Jordan row factors
 __shared__ int s_piv;                             // NaN mode: pivot row
+__shared__ int s_prow[3];  // block permutation, held-out sample: the permuted block's features [lo, hi) and their row
 
 // The fit the calling CTA runs, and its workspace: the fit in per-fit mode, the CTA's slot in slot mode.  Derived again where
 // needed rather than held in registers through the component loop (the kernel has none to spare).
@@ -105,6 +116,18 @@ __device__ __forceinline__ size_t sf_cur_ws(const mbpls_smallfit_args& a) { retu
 // holds it through the fit).
 __device__ __forceinline__ double* sf_flag(const mbpls_smallfit_args& a) {
   return a.small + (static_cast<size_t>(sf_cur_fit(a)) + 1) * (static_cast<size_t>(a.K) * (a.q + 2 * a.B + 4) + a.B + 2) - 1;
+}
+
+// Block permutation: the row map of fit f (perm_rows row r for fit_perm[f] = (r, b)) and the feature range [*lo, *hi) of
+// block b, read through off (the block offsets); NULL and an empty range for a fit that permutes nothing.  Derived where it is
+// used, like sf_cur_fit.
+__device__ __forceinline__ const int* sf_block_map(const mbpls_smallfit_args& a, int f, const int* off, int* lo, int* hi) {
+  *lo = *hi = 0;
+  if (!a.fit_perm || a.fit_perm[2 * f] < 0) return nullptr;
+  const int b = a.fit_perm[2 * f + 1];
+  *lo = off[b];
+  *hi = off[b + 1];
+  return a.perm_rows + static_cast<size_t>(a.fit_perm[2 * f]) * a.n_src;
 }
 
 // One whole fit by the calling CTA: inputs and outputs (small, beta, fit_preds) of fit sf_cur_fit, workspace sf_cur_ws.
@@ -153,15 +176,20 @@ __device__ __forceinline__ void sf_fit(const mbpls_smallfit_args& a) {
   for (int b = tid; b <= B; b += SF_THREADS) s_off[b] = a.block_off[b];
   __syncthreads();
 
-  // ---- prologue: gather + StandardScaler (mbpls.py:303-326), varx / vary (:822-830)
-  for (int j = warp; j < p; j += SF_WARPS) {
-    const double z2 = sf_ingest_feature<NANMODE>(a.Xsrc + static_cast<size_t>(j) * a.ldx, tr, ntr,
-                                                 Xw + static_cast<size_t>(j) * ldw, a.standardize, xmean + j, xvar + j,
-                                                 xscale + j, xobs + j, lane);
-    if (lane == 0) xzss[j] = z2;
+  // ---- prologue: gather + StandardScaler (mbpls.py:303-326), varx / vary (:822-830); the features of a permuted block
+  // read their rows through its map (the census of NaN mode below is taken on this copy, so the holes move with the rows)
+  {
+    int plo, phi;
+    const int* pmap = sf_block_map(a, f, s_off, &plo, &phi);
+    for (int j = warp; j < p; j += SF_WARPS) {
+      const double z2 = sf_ingest_feature<NANMODE>(a.Xsrc + static_cast<size_t>(j) * a.ldx, tr, j >= plo && j < phi ? pmap : nullptr,
+                                                   ntr, Xw + static_cast<size_t>(j) * ldw, a.standardize, xmean + j, xvar + j,
+                                                   xscale + j, xobs + j, lane);
+      if (lane == 0) xzss[j] = z2;
+    }
   }
   for (int c = warp; c < q; c += SF_WARPS) {
-    const double z2 = sf_ingest_feature<NANMODE>(a.Ysrc + static_cast<size_t>(c) * a.ldx, ytr, ntr,
+    const double z2 = sf_ingest_feature<NANMODE>(a.Ysrc + static_cast<size_t>(c) * a.ldx, ytr, nullptr, ntr,
                                                  Yw + static_cast<size_t>(c) * ldw, a.standardize, ymean + c, yvar + c,
                                                  yscale + c, yobs + c, lane);
     if (lane == 0) yzss[c] = z2;
@@ -635,10 +663,21 @@ __device__ __forceinline__ void sf_fit(const mbpls_smallfit_args& a) {
   // y_hat_k(x) = sum_{j<=k} (z . r_j) v_j, z the standardised sample; back to the Y scale (:1386)
   for (int t = 0; t < nte; ++t) {
     const int idx = te[t];
+    if (a.fit_perm) {  // a permuted block's features of the held-out sample come from its mapped row (kept in shared memory:
+                       // the NaN instantiation has no register to spare here)
+      if (tid == 0) {
+        int lo, hi;
+        const int* m = sf_block_map(a, fit, s_off, &lo, &hi);
+        s_prow[0] = lo;
+        s_prow[1] = hi;
+        s_prow[2] = m ? m[idx] : idx;
+      }
+      __syncthreads();
+    }
     for (int k = warp; k < K; k += SF_WARPS) {
       double s = 0.0;
       for (int j = lane; j < p; j += 32) {
-        double z = a.Xsrc[static_cast<size_t>(j) * a.ldx + idx];
+        double z = a.Xsrc[static_cast<size_t>(j) * a.ldx + (a.fit_perm && j >= s_prow[0] && j < s_prow[1] ? s_prow[2] : idx)];
         if (a.standardize) z = (z - xmean[j]) / xscale[j];
         if constexpr (NANMODE) {  // NaN counts as zero after scaling (:1379-1384); s_part[k] = z . w_k
           if (isnan(z)) z = 0.0;
@@ -722,6 +761,17 @@ int mbpls_smallfit_nipals_f64(const mbpls_smallfit_args* a, void* stream) {
                               : mbpls_smallfit_scratch_doubles(a->p, a->B, a->ldw);
   if (need < 0 || a->scratch_stride < need) return MBPLS_ERR_ARG;
   const cudaStream_t st = static_cast<cudaStream_t>(stream);
+  if (a->perm_rows || a->fit_perm) {  // block permutation: every (r, b) pair must name a row of perm_rows and a block
+    if (!a->perm_rows || !a->fit_perm || !a->train_idx || a->n_perm < 1) return MBPLS_ERR_ARG;
+    std::vector<int> pairs(2 * static_cast<size_t>(a->nfits));
+    cudaError_t e = cudaMemcpyAsync(pairs.data(), a->fit_perm, pairs.size() * sizeof(int), cudaMemcpyDeviceToHost, st);
+    if (e == cudaSuccess) e = cudaStreamSynchronize(st);
+    if (e != cudaSuccess) return MBPLS_CUDA_ERR(e);
+    for (int f = 0; f < a->nfits; ++f) {
+      const int r = pairs[2 * f], b = pairs[2 * f + 1];
+      if (r < -1 || r >= a->n_perm || (r >= 0 && (b < 0 || b >= a->B))) return MBPLS_ERR_ARG;
+    }
+  }
   if (a->nslots > 0) {
     const cudaError_t e = cudaMemsetAsync(a->ticket, 0, sizeof(int), st);
     if (e != cudaSuccess) return MBPLS_CUDA_ERR(e);

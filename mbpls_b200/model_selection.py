@@ -15,7 +15,9 @@ Validation of a fitted model's reported quantities: ``permutation_test_score`` (
 the cross-validation re-run on permutations of ``y``) and ``bootstrap`` (how stable are ``A_`` / ``beta_``? refits on
 resamples of the rows).  Both need 10^3 - 10^5 fits; for NIPALS, dense or with missing values (``sparse_data=True``), they
 all run in one slot-mode launch of ``smallfit_kernel`` (persistent CTAs that claim fit after fit, X rows paired with permuted /
-resampled Y rows on the device).
+resampled Y rows on the device).  ``block_permutation_test`` asks whether each block adds anything given the others: it
+permutes the rows of one block at a time and re-runs the cross-validation and the fit on all rows, for null distributions of
+the score and of the block's importance ``A_``; in the batch, a fit reads the permuted block's columns through a row map.
 """
 from __future__ import annotations
 
@@ -31,7 +33,7 @@ from . import smallfit as SF
 from .engine import F64
 from .mbpls import MBPLS, _as_2d_source, _is_block_list
 
-__all__ = ["cross_val_predict", "permutation_test_score", "bootstrap"]
+__all__ = ["cross_val_predict", "permutation_test_score", "bootstrap", "block_permutation_test"]
 
 
 def _folds(n: int, cv) -> list:
@@ -70,19 +72,27 @@ def _prefix_betas(model: MBPLS, ks: Sequence[int], device) -> list:
 
 def _fold_predictions(estimator, Xraw, Yraw, shard, q, K, ks, fits, device) -> list:
     """One refit through ``MBPLS.fit`` per (X train rows, Y train rows, test rows) of ``fits``, on the feature-major device
-    copies Xraw / Yraw.  Returns, per fit, {k: (len(test rows), q) array} of held-out predictions (k in ks, or K)."""
+    copies Xraw / Yraw.  A fit may carry a fourth entry (b, pi): the columns of block b then come from rows pi[train rows] and
+    pi[test rows] (a block permutation test).  Returns, per fit, {k: (len(test rows), q) array} of held-out predictions (k in
+    ks, or K)."""
     off = shard.block_off
     out = []
-    for tr, ytr, te in fits:
-        tr_d = torch.as_tensor(np.asarray(tr), device=device, dtype=torch.long)
-        ytr_d = tr_d if ytr is tr else torch.as_tensor(np.asarray(ytr), device=device, dtype=torch.long)
-        te_d = torch.as_tensor(np.asarray(te), device=device, dtype=torch.long)
+    rows = lambda idx: torch.as_tensor(np.asarray(idx), device=device, dtype=torch.long)
+    for fit in fits:
+        tr, ytr, te = fit[:3]
+        tr_d = rows(tr)
+        ytr_d = tr_d if ytr is tr else rows(ytr)
+        te_d = rows(te)
         ntr, nte = len(tr), len(te)
         Xtr = E.alloc_feature_major(shard.p_local, ntr, device)
         Xtr[:, :ntr] = Xraw.index_select(1, tr_d)              # gather of the training samples (device copy)
         Ytr = Yraw.index_select(1, ytr_d).t().contiguous()     # ntr x q
         Xte = E.alloc_feature_major(shard.p_local, nte, device)
         Xte[:, :nte] = Xraw.index_select(1, te_d)
+        if len(fit) > 3:                                       # block b's columns on the permuted rows
+            b, pi = fit[3]
+            Xtr[off[b]:off[b + 1], :ntr] = Xraw[off[b]:off[b + 1]].index_select(1, rows(pi[tr]))
+            Xte[off[b]:off[b + 1], :nte] = Xraw[off[b]:off[b + 1]].index_select(1, rows(pi[te]))
         m = clone(estimator)
         m.set_params(n_components=K, copy=False)
         m.set_runtime(device=device, materialize=False)
@@ -131,10 +141,10 @@ def _require_finite(arrays, allow_nan: bool = False):
             raise ValueError("Input contains NaN or infinity.")
 
 
-def _nan_eligible(blocks, Ysrc, x_rows, y_rows) -> np.ndarray:
+def _nan_eligible(blocks, Ysrc, x_rows, y_rows, block_cols=None, block_rows=None) -> np.ndarray:
     """smallfit.nan_fits_eligible on the source arrays: per fit, True if the NaN-mode batch can run it."""
     x_obs = np.hstack([SF.observed(b) for b in blocks])
-    return SF.nan_fits_eligible(x_obs, SF.observed(Ysrc), x_rows, y_rows)
+    return SF.nan_fits_eligible(x_obs, SF.observed(Ysrc), x_rows, y_rows, block_cols, block_rows)
 
 
 def _upload(blocks, Ysrc, n, q, shard, device):
@@ -434,12 +444,7 @@ def bootstrap(estimator: MBPLS, X, y, n_resamples: int = 100, random_state=0) ->
                     for name in names:
                         res[name][r] = attrs[name]
     for r in redo:
-        m = clone(estimator)
-        m.set_runtime(**rt)
-        t = lambda a: a[torch.as_tensor(idx[r], device=a.device)] if isinstance(a, torch.Tensor) else a[idx[r]]
-        with warnings.catch_warnings():
-            warnings.simplefilter("ignore")
-            m.fit([t(b) for b in blocks], t(Ysrc).reshape(-1) if y1d else t(Ysrc))
+        m = _refit(estimator, rt, blocks, Ysrc, y1d, idx[r])
         for name in names:
             res[name][r] = getattr(m, name)
     out = {"indices": idx}
@@ -447,3 +452,151 @@ def bootstrap(estimator: MBPLS, X, y, n_resamples: int = 100, random_state=0) ->
     if "n_iter_" in out:
         out["n_iter_"] = out["n_iter_"].astype(np.int64)
     return out
+
+
+def _refit(estimator, rt, blocks, Ysrc, y1d, rows, block_perm=None, n_components=None) -> MBPLS:
+    """``clone(estimator)`` with the runtime options ``rt`` fitted through ``MBPLS.fit`` on rows ``rows`` of every block and of
+    y.  block_perm (b, pi): block b takes the rows pi[rows] instead."""
+    m = clone(estimator)
+    if n_components is not None:
+        m.set_params(n_components=n_components)
+    m.set_runtime(**rt)
+    t = lambda a, r: a[torch.as_tensor(r, device=a.device)] if isinstance(a, torch.Tensor) else a[r]
+    Xb = [t(x, block_perm[1][rows] if block_perm is not None and b == block_perm[0] else rows) for b, x in enumerate(blocks)]
+    with warnings.catch_warnings():
+        warnings.simplefilter("ignore")
+        m.fit(Xb, t(Ysrc, rows).reshape(-1) if y1d else t(Ysrc, rows))
+    return m
+
+
+def block_permutation_test(estimator: MBPLS, X, y, cv=5, n_permutations: int = 100, random_state=0, scoring=None,
+                           n_components_list: Optional[Iterable[int]] = None) -> dict:
+    """Does block b add anything, given the other blocks?  A permutation test of each block of a multiblock model: the rows of
+    block b alone are permuted, which breaks its link with ``y`` and with the other blocks and leaves everything else as it
+    is; the cross-validation is run again, and the model refitted on all rows.
+
+    ``estimator`` is an unfitted ``mbpls_b200.MBPLS`` and ``X`` a list of B >= 2 blocks (one array: see
+    ``permutation_test_score``).  The R = ``n_permutations`` row orders are drawn as ``permutation_test_score`` draws them
+    (``check_random_state(random_state)``, then ``permutation(n)`` R times), and the same R orders permute every block, so the
+    blocks' null distributions are paired.  The folds are taken from ``cv`` once; ``scoring`` takes the values of
+    ``permutation_test_score``.  Returns a dict:
+
+    - ``score``: the mean over the folds of the unpermuted cross-validated score;
+    - ``permutation_scores`` (B, R): the same with the rows of block b permuted by permutation r;
+    - ``pvalue`` (B,): ``(#{permutation_scores[b] >= score} + 1) / (R + 1)``;
+    - ``A_`` (B, K): ``A_`` of the unpermuted fit on all rows (block b's importance in component k);
+    - ``A_permuted`` (B, R, K): block b's row of ``A_`` in the fits on all rows with block b permuted by permutation r;
+    - ``A_pvalue`` (B, K): ``(#{A_permuted[b, :, k] >= A_[b, k]} + 1) / (R + 1)``.
+
+    With ``n_components_list``, ``score``, ``permutation_scores`` and ``pvalue`` are dicts keyed by k from one ``max(k)``-component
+    fit per fold, permutation and block, and the ``A_*`` entries are those of the ``max(k)`` fit (``A_[:, :k]`` is the
+    k-component model's: a NIPALS component does not depend on later ones).  SIMPLS computes no ``A_``: the ``A_*`` keys are
+    absent then.
+
+    NIPALS problems small enough for one CTA, dense or with ``sparse_data=True``, run every fit (the cross-validations, the
+    unpermuted fit on all rows and the B x R block-permuted ones) in one kernel launch; other methods, larger problems and the
+    fits the batch cannot run (more components than rank; with missing values, rows that leave a feature or Y column
+    unobserved or no Y column fully observed) refit through ``MBPLS.fit``.
+    """
+    _check_scoring(scoring)
+    rt = estimator._runtime()
+    if rt["group"] is not None:
+        raise NotImplementedError("block_permutation_test runs on one GPU: no process group in the runtime options")
+    if not (isinstance(X, list) and len(X) >= 2 and _is_block_list(X)):
+        raise ValueError("block_permutation_test needs X as a list of at least two blocks; permutation_test_score tests a "
+                         "single array")
+    device = E.require_cuda(rt["device"])
+    blocks, Ysrc, y1d, n, q, sizes = _sources(X, y)
+    ks = None if n_components_list is None else sorted(set(int(k) for k in n_components_list))
+    K = estimator.n_components if ks is None else max(ks)
+    kk, B = ks or [K], len(sizes)
+    folds = _folds(n, cv)
+    perms = _permutations(n, int(n_permutations), random_state)[1:]  # R x n, without the identity
+    R, nf = perms.shape[0], len(folds)
+    units = [None] + [(b, r) for b in range(B) for r in range(R)]   # unit 0 permutes nothing, unit 1 + b R + r block b by r
+    has_A = estimator.method != 'SIMPLS' or bool(estimator.sparse_data)
+    ld_t = max(1, max(len(te) for _, te in folds))
+    preds = np.full((len(units), nf, len(kk), ld_t, q), np.nan)      # held-out predictions by position in the fold's test list
+    A_all = np.full((len(units), B, K), np.nan)                      # A_ of the fits on all rows
+
+    with torch.cuda.device(device):
+        shard = E.ShardMap.build(sizes, 0, 1)
+        redo_cv, redo_full = [(u, i) for u in range(len(units)) for i in range(nf)], list(range(len(units)) if has_A else [])
+        if SF.batch_eligible(estimator, n, sum(sizes)):
+            redo_cv, redo_full = _block_permutation_batches(estimator, blocks, Ysrc, n, q, shard, K, kk, folds, perms, units,
+                                                            preds, A_all, device)
+        if redo_cv:  # every CV fit (generic path), or those the batch flagged or could not run, one by one through MBPLS.fit
+            Xraw, Yraw = _upload(blocks, Ysrc, n, q, shard, device)
+            todo = []
+            for u, i in redo_cv:
+                tr, te = folds[i]
+                todo.append((tr, tr, te) if units[u] is None else (tr, tr, te, (units[u][0], perms[units[u][1]])))
+            for (u, i), pred in zip(redo_cv, _fold_predictions(estimator, Xraw, Yraw, shard, q, K, kk, todo, device)):
+                for j, k in enumerate(kk):
+                    preds[u, i, j, :len(folds[i][1])] = pred[k]
+    for u in redo_full:
+        bp = None if units[u] is None else (units[u][0], perms[units[u][1]])
+        A_all[u] = _refit(estimator, rt, blocks, Ysrc, y1d, np.arange(n), bp, n_components=K).A_
+
+    Yh = _host(Ysrc)
+    S = np.zeros((len(units), len(kk)))
+    for i, (_, te) in enumerate(folds):
+        S += _scores(scoring, Yh[te][None, None], preds[:, i, :, :len(te)])
+    return _block_permutation_result(S / nf, A_all if has_A else None, B, R, ks)
+
+
+def _block_permutation_result(S: np.ndarray, A_all: Optional[np.ndarray], B: int, R: int, ks) -> dict:
+    """block_permutation_test's dict from the mean fold scores S ((1 + B R) units x prefix models, unit 0 unpermuted, unit
+    1 + b R + r block b permuted by permutation r) and the A_ of the fits on all rows (units x B x K, None: no A_)."""
+    res = {}
+    for j, k in enumerate(ks or [None]):
+        score, perm_scores = float(S[0, j]), S[1:, j].reshape(B, R)
+        res[k] = (score, perm_scores, (np.sum(perm_scores >= score, axis=1) + 1.0) / (R + 1.0))
+    out = {name: (res[None][i] if ks is None else {k: v[i] for k, v in res.items()})
+           for i, name in enumerate(("score", "permutation_scores", "pvalue"))}
+    if A_all is not None:
+        A0 = A_all[0]
+        Ap = np.stack([A_all[1 + b * R:1 + (b + 1) * R, b] for b in range(B)])  # B x R x K
+        out.update(A_=A0, A_permuted=Ap, A_pvalue=(np.sum(Ap >= A0[:, None, :], axis=1) + 1.0) / (R + 1.0))
+    return out
+
+
+def _block_permutation_batches(estimator, blocks, Ysrc, n, q, shard, K, kk, folds, perms, units, preds, A_all, device):
+    """Every fit of a block permutation test in slot-mode launches of smallfit_kernel (one unless the per-fit outputs exceed
+    CV_WORKSPACE_BYTES).  Per unit (no permutation, or block b permuted by permutation r): the fold fits, which gather X rows
+    tr_i (block b's columns through the row map) and predict X rows te_i for every prefix model, then one fit on all rows.
+    Fills preds and A_all; returns the (unit, fold) pairs and the units of the fits on all rows that were flagged or, with
+    sparse_data=True, not eligible (smallfit.nan_fits_eligible), which the caller refits through MBPLS.fit."""
+    from .mbpls import _check_limits
+    rt = estimator._runtime()
+    sparse = bool(estimator.sparse_data)
+    _check_limits(K, q, len(shard.sizes))
+    _require_finite(blocks + [Ysrc], allow_nan=sparse)
+    nf, U, off = len(folds), len(units), shard.block_off
+    per = nf + 1                                                     # fits per unit: the folds, then all rows
+    trs = [np.asarray(tr, dtype=np.int32) for tr, _ in folds] + [np.arange(n, dtype=np.int32)]
+    tes = [np.asarray(te, dtype=np.int32) for _, te in folds] + [np.zeros(0, dtype=np.int32)]
+    pair = lambda u: (-1, 0) if units[u] is None else (units[u][1], units[u][0])  # (r, b) as the kernel takes it
+    redo = set()
+    if sparse:
+        cols = [None if v is None else (off[v[0]], off[v[0] + 1]) for v in units for _ in trs]
+        prow = [None if v is None else perms[v[1]][t] for v in units for t in trs]
+        ok = _nan_eligible(blocks, Ysrc, [t for _ in units for t in trs], [t for _ in units for t in trs], cols, prow)
+        redo.update(divmod(int(f), per) for f in np.flatnonzero(~ok))
+    D, n, sizes, p, q, ldx = SF.pack_source(blocks, Ysrc, device)
+    B, ld_t = len(sizes), preds.shape[3]
+    kidx = [k - 1 for k in kk]
+    small_sz = K * (q + 2 * B + 4) + B + 2
+    for u0, u1 in SF.unit_batches(U, per, 8 * (small_sz + K * ld_t * q)):
+        F = (u1 - u0) * per
+        lay, out, fp, keep = SF.launch(
+            D, n, p, q, ldx, off, K, bool(estimator.standardize), E.norm_kind_of(estimator.nipals_convergence_norm),
+            estimator.max_tol, rt["max_iter"], [t for _ in range(u0, u1) for t in trs], [t for _ in range(u0, u1) for t in tes],
+            nslots=SF.slot_count(device, F), fit_preds=True, want_beta=False, nanmode=sparse,
+            block_perm=(perms if len(perms) else np.zeros((1, n), np.int32), [pair(u) for u in range(u0, u1) for _ in trs]))
+        small = E.to_host(lay.section(out, "small")).reshape(u1 - u0, per, -1)
+        host = E.to_host(fp).reshape(u1 - u0, per, K, -1, q)         # fits x K x ld_t x q
+        preds[u0:u1] = host[:, :nf][:, :, kidx]
+        A_all[u0:u1] = small[:, nf, K * q:K * q + K * B].reshape(u1 - u0, K, B).transpose(0, 2, 1)
+        redo.update((u0 + int(u), int(i)) for u, i in zip(*np.nonzero(small[:, :, -1] != 0.0)))
+    return sorted((u, i) for u, i in redo if i < nf), sorted(u for u, i in redo if i == nf)

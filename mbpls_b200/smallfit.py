@@ -54,20 +54,30 @@ def batch_eligible(estimator, ntr_max: int, p: int) -> bool:
     return True
 
 
-def nan_fits_eligible(x_obs: np.ndarray, y_obs: np.ndarray, x_rows: Sequence, y_rows: Sequence) -> np.ndarray:
+def nan_fits_eligible(x_obs: np.ndarray, y_obs: np.ndarray, x_rows: Sequence, y_rows: Sequence,
+                      block_cols: Optional[Sequence] = None, block_rows: Optional[Sequence] = None) -> np.ndarray:
     """Per fit, whether the NaN-mode batch runs it (True) or it goes to MBPLS.fit (False).
 
     x_obs (n, p) / y_obs (n, q): True where the source holds a value (not NaN); x_rows[f] / y_rows[f]: the X rows of fit f and
-    the Y rows paired with them (repeats allowed).  A fit needs an observed value of every feature and every Y column on its
-    rows, and a Y column observed on all of its Y rows to start the Y scores from (mbpls.py:832-836; without one the reference
-    draws np.random.rand)."""
+    the Y rows paired with them (repeats allowed).  block_cols[f] None, or a column range (lo, hi) of X that fit f reads on the
+    rows block_rows[f] instead of x_rows[f] (a block-permuted fit).  A fit needs an observed value of every feature and every Y
+    column on its rows, and a Y column observed on all of its Y rows to start the Y scores from (mbpls.py:832-836; without one
+    the reference draws np.random.rand)."""
     def counts(obs, rows):  # (fits, columns): observed values on each fit's rows, with multiplicity
         n = obs.shape[0]
         lens = np.fromiter((len(r) for r in rows), dtype=np.int64, count=len(rows))
         flat = np.concatenate([np.asarray(r, dtype=np.int64) for r in rows]) if len(rows) else np.zeros(0, np.int64)
         mult = np.bincount(np.repeat(np.arange(len(rows)), lens) * n + flat, minlength=len(rows) * n).reshape(len(rows), n)
         return mult.astype(np.float64) @ obs.astype(np.float64), lens  # exact counts, through BLAS
-    xc, _ = counts(np.asarray(x_obs, dtype=bool), x_rows)
+    x_obs = np.asarray(x_obs, dtype=bool)
+    xc, _ = counts(x_obs, x_rows)
+    if block_cols is not None:
+        groups = {}
+        for f, c in enumerate(block_cols):
+            if c is not None:
+                groups.setdefault((int(c[0]), int(c[1])), []).append(f)
+        for (lo, hi), fs in groups.items():
+            xc[fs, lo:hi] = counts(x_obs[:, lo:hi], [block_rows[f] for f in fs])[0]
     yc, ylen = counts(np.asarray(y_obs, dtype=bool), y_rows)
     return (xc > 0).all(axis=1) & (yc > 0).all(axis=1) & (yc == ylen[:, None]).any(axis=1)
 
@@ -164,16 +174,20 @@ class Layout:
 def launch(D: torch.Tensor, n_src: int, p: int, q: int, ldx: int, block_off: Sequence[int], K: int, standardize: bool,
            norm_kind: int, max_tol: float, max_iter: int, train_sets: Optional[List[np.ndarray]],
            test_sets: Optional[List[np.ndarray]] = None, *, y_sets: Optional[List[np.ndarray]] = None, nslots: int = 0,
-           fit_preds: bool = False, want_beta: bool = True, nanmode: bool = False):
+           fit_preds: bool = False, want_beta: bool = True, nanmode: bool = False, block_perm=None):
     """Run ``len(train_sets)`` fits concurrently (train_sets None: one fit on all samples).  ``D`` is pack_source's buffer.
     y_sets: per fit, the Y rows paired with its X rows train_sets[f] (None: the same rows).  nslots > 0: slot mode, that many
     persistent CTAs work through the fits, workspace per slot (nslots 0: one CTA and one workspace per fit).  fit_preds: the
     held-out predictions per fit, (nfits, K, max test size, q), instead of by sample (K, n_src, q; not in slot mode).
     want_beta False: no beta section (slot mode only).  nanmode: the NaN-mode fit of sparse_data=True (K <= 64); a fit the
-    kernel cannot run (see nan_fits_eligible) comes back flagged like a singular one.
+    kernel cannot run (see nan_fits_eligible) comes back flagged like a singular one.  block_perm: (perm_table (R, n_src) row
+    permutations, pairs (nfits, 2)): a fit with pairs[f] = (r, b), r >= 0, reads every X row i of block b (training and held-out
+    rows) from row perm_table[r, i]; r = -1 permutes nothing (not with train_sets None).
     Returns (layout, packed device result buffer, predictions device tensor or None, buffers to keep alive)."""
     dev = D.device
     B = len(block_off) - 1
+    if block_perm is not None and train_sets is None:
+        raise ValueError("block_perm needs train_sets")
     boff_ptr = C.c_void_p(D.data_ptr() + 8 * (p + q) * ldx)  # the table pack_source put behind the matrix
     packed = None
     if train_sets is None:  # one fit on every sample of the source: no index tables at all
@@ -199,12 +213,16 @@ def launch(D: torch.Tensor, n_src: int, p: int, q: int, ldx: int, block_off: Seq
             ints += table(test_sets, ld_t)
         if y_sets is not None:
             ints.append(table(y_sets, ld_idx)[0])
+        if block_perm is not None:
+            ints += [np.ascontiguousarray(block_perm[0], dtype=np.int32).ravel(),
+                     np.ascontiguousarray(block_perm[1], dtype=np.int32).ravel()]
         if nslots:
             ints.append(np.zeros(1, dtype=np.int32))  # the ticket counter (zeroed again on the stream by the entry point)
         packed = torch.from_numpy(np.concatenate(ints)).to(dev, non_blocking=True)  # every index table in one copy
         offs = np.cumsum([0] + [len(a) for a in ints])
         iptr = lambda i: C.c_void_p(packed.data_ptr() + 4 * int(offs[i]))
-    nt = 4 if test_sets is not None else 2  # tables before the Y rows and the ticket
+    nt = 4 if test_sets is not None else 2  # tables before the Y rows, the block permutations and the ticket
+    npm = nt + (y_sets is not None)  # the permutation table, then the (r, b) pairs
     S = nslots or F  # workspaces
     lay = Layout(F, p, q, B, K, ldw, nslots, want_beta)
     out = torch.empty(lay.total, dtype=F64, device=dev)
@@ -227,7 +245,10 @@ def launch(D: torch.Tensor, n_src: int, p: int, q: int, ldx: int, block_off: Seq
         Ts=sec("Ts"), U=sec("U"), Tb=sec("Tb"), small=sec("small"), R=sec("R"), beta=sec("beta") if want_beta else None,
         preds=preds.data_ptr() if preds is not None and not fit_preds else None, scratch=scratch.data_ptr(), scratch_stride=sstride,
         ytrain_idx=iptr(nt) if y_sets is not None else None, fit_preds=preds.data_ptr() if fit_preds and preds is not None else None,
-        nslots=int(nslots), ticket=iptr(len(ints) - 1) if nslots else None, nanmode=1 if nanmode else 0)
+        nslots=int(nslots), ticket=iptr(len(ints) - 1) if nslots else None, nanmode=1 if nanmode else 0,
+        perm_rows=iptr(npm) if block_perm is not None else None,
+        n_perm=int(np.shape(block_perm[0])[0]) if block_perm is not None else 0,
+        fit_perm=iptr(npm + 1) if block_perm is not None else None)
     call("mbpls_smallfit_nipals_f64", C.byref(args), stream_ptr(dev))
     return lay, out, preds, (packed, work, scratch)
 
